@@ -63,7 +63,38 @@ def parse():
                     help="host staging buffers of the e2e run: torch pinned memory, or write-combined pinned memory (uyd_host_alloc)")
     ap.add_argument("--sustain", type=float, default=2.0, metavar="SECONDS",
                     help="also run the resident step back to back for at least this long, with clocks (0 = skip)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="write what the last timed step returned (rank 0: detections and counts) as DIR/<name>.npy, "
+                         "so that two builds can be compared output for output on the same seeded inputs")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl == "reference":
+        ap.error("--dump-outputs applies to the GPU path only")
+    return a
+
+
+DUMP_BYTES = 64_000_000   # --dump-outputs writes at most this much data
+
+
+def dump_outputs(out_dir: str, arrays: dict) -> None:
+    """One float32 / float64 .npy file per returned array (float32 data as is, integer data widened to float64,
+    which holds every int32 exactly).  The arrays share their leading (image) dimension; where all images would take
+    more than DUMP_BYTES, a fixed seeded sample of them is written, with their indices as image_index.npy."""
+    import numpy as np
+
+    out = {k: t.detach().cpu() for k, t in arrays.items()}
+    out = {k: t if t.dtype == torch.float32 else t.double() for k, t in out.items()}
+    n = next(iter(out.values())).shape[0]
+    per_image = sum(t[0].numel() * t.element_size() for t in out.values())
+    if n * per_image > DUMP_BYTES:
+        keep = torch.randperm(n, generator=torch.Generator().manual_seed(0))[: DUMP_BYTES // (per_image + 8)].sort().values
+        out = {k: t[keep] for k, t in out.items()}
+        out["image_index"] = keep.double()
+    d = Path(out_dir)
+    d.mkdir(parents=True, exist_ok=True)
+    for name, t in out.items():
+        np.save(d / f"{name}.npy", t.numpy())
 
 
 def peaks():
@@ -390,8 +421,10 @@ def main():
     det_host = torch.empty(B, MAX_DET, 6).pin_memory()
     cnt_host = torch.empty(B, dtype=torch.int32).pin_memory()
 
+    last = []   # what the most recent resident step returned (det, cnt): --dump-outputs writes the last timed one
+
     def step_resident():
-        return model.predict_batched(x_dev, CONF, IOU, MAX_DET)
+        last[:] = model.predict_batched(x_dev, CONF, IOU, MAX_DET)
 
     def step_e2e():  # one blocking call: H2D, compute, D2H serialised
         x_u8.copy_(x_host, non_blocking=True)
@@ -453,7 +486,7 @@ def main():
     ms = plan.profile(x_dev, y_prof)
     top = max(range(len(ms)), key=lambda i: ms[i])
     top_text, top_flops, top_bytes = plan.op_info(top)
-    plan.set_timed_op(top, a.steps)
+    plan.set_timed_op(top, min(a.steps, 4096))   # the library keeps at most 4096 event pairs: longer runs sample the first ones
 
     def timed(fn, steps):
         if world > 1:
@@ -480,6 +513,8 @@ def main():
         sampler.join(timeout=10)   # an nvidia-smi query still in flight stalls work submission for tens of ms
     top_ms_total, top_n = plan.timed_op_read()
     plan.set_timed_op(-1, 0)
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, {"detections": last[0], "counts": last[1]})
 
     def run_resident_stream(steps):  # the streaming API on resident frames: NMS of step i on a second stream under step i + 1
         for _det, _cnt in model.predict_stream((x_dev for _ in range(steps)), CONF, IOU, MAX_DET, to_host=False):

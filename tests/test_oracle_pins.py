@@ -14,16 +14,21 @@ from oracle import postproc as pp
 from oracle import yolo_graph as yg
 
 sys.path.insert(0, str(GOLDEN))
-import make_golden  # noqa: E402  (only its pure-python case table is used)
+import make_golden  # noqa: E402  (only its pure-python case table and GOLDEN_THREADS are used)
 
 
 @pytest.mark.parametrize("bc", [8, 32])
 def test_custom_graph_matches_golden_from_real_model_py(bc):
     g = np.load(GOLDEN / f"custom_bc{bc}.npz")
-    net = oi.build_custom(seed=7, base_channels=bc, calib_batch=2, size=int(g["size"]))
-    assert oi.state_dict_sha256(net.state_dict()) == str(g["sha256"]), "seeded weights drifted from the fixture"
-    with torch.no_grad():
-        outs = net(oi.seeded_frames(1, int(g["size"]), seed=11))
+    saved = torch.get_num_threads()
+    torch.set_num_threads(make_golden.GOLDEN_THREADS)   # the count custom_bc*.npz were computed with
+    try:
+        net = oi.build_custom(seed=7, base_channels=bc, calib_batch=2, size=int(g["size"]))
+        assert oi.state_dict_sha256(net.state_dict()) == str(g["sha256"]), "seeded weights drifted from the fixture"
+        with torch.no_grad():
+            outs = net(oi.seeded_frames(1, int(g["size"]), seed=11))
+    finally:
+        torch.set_num_threads(saved)
     for lvl, (c, r) in zip((2, 3, 4), outs):
         np.testing.assert_array_equal(c.numpy(), g[f"p{lvl}_cls"])
         np.testing.assert_array_equal(r.numpy(), g[f"p{lvl}_reg"])
