@@ -20,6 +20,8 @@
  *   uyd_nms                 <- Ultralytics non_max_suppression + torchvision.ops.nms
  *                              (train.py:396-405) and run_gpu_nms + copy_valid_detections_to_host
  *                              (gpu_postprocess.h:70-78)
+ *   uyd_nms_tlbr            <- decode_yolo_head x3 + run_gpu_nms of a whole batch in one launch
+ *                              (perception_node.cpp:581-689)
  */
 #ifndef UYD_H
 #define UYD_H
@@ -296,6 +298,20 @@ int uyd_nms_detections(uyd_ctx *ctx, const uyd_detection *dets, const int *cell_
  * d_out_count (device, may be NULL) receives the number of survivors. */
 int uyd_nms_detections_inplace(uyd_ctx *ctx, uyd_detection *dets, const int *cell_idx, int n, float iou_thr,
                                int *d_out_count, uyd_stream stream);
+
+/* TLBR decode (postprocess.hpp:94-145) + class-aware greedy NMS (postprocess.hpp:44-67) of a whole batch in ONE
+ * launch.  heads[l]: [batch, grid_h[l], grid_w[l], num_classes + 4] fp32 (class logits, then l, t, r, b distances).
+ * Ties in confidence resolve to the lower cell index (levels numbered consecutively in the given order).
+ * max_nms > 0: only the max_nms best candidates per image enter the NMS.  out_det [batch, max_det, 6]
+ * (x1,y1,x2,y2,conf,cls), out_count [batch]; every element written.  max_det <= 1024.
+ * Per cell, the same statement as uyd_decode_tlbr (conf_thr, conformal_q, strict), so the rows equal those of
+ * uyd_decode_tlbr per level followed by uyd_nms_detections.  heads, grid_h, grid_w and strides are host arrays of nl
+ * entries.  Nothing is launched and UYD_E_ARG is returned for nl < 1, a NULL pointer, a non-positive batch, class
+ * count, grid size or stride, max_nms < 0 or a head not aligned to a float; UYD_E_UNSUPPORTED for nl > 8, max_det
+ * outside [1, 1024] or 2^31 cells or more per image.  No host synchronisation. */
+int uyd_nms_tlbr(uyd_ctx *ctx, const float *const *heads, const int *grid_h, const int *grid_w, const int *strides,
+                 int nl, int batch, int num_classes, float conf_thr, float conformal_q, int strict, float iou_thr,
+                 int max_nms, int max_det, float *out_det, int *out_count, uyd_stream stream);
 
 /* Ordered compaction of the valid records among the first n (<= 1024) into `out` + their number (device):
  * the cub::DeviceSelect::If of copy_valid_detections_to_host (gpu_postprocess.cu:412-416). */

@@ -117,6 +117,9 @@ SIGNATURES = {
     "uyd_nms_detections": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_float, C.c_void_p,
                                      C.c_size_t, C.c_void_p, C.c_void_p, C.c_void_p]),
     "uyd_nms_detections_inplace": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_float, C.c_void_p, C.c_void_p]),
+    "uyd_nms_tlbr": (C.c_int, [C.c_void_p, C.POINTER(C.c_void_p), C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(C.c_int),
+                               C.c_int, C.c_int, C.c_int, C.c_float, C.c_float, C.c_int, C.c_float, C.c_int, C.c_int,
+                               C.c_void_p, C.c_void_p, C.c_void_p]),
     "uyd_compact_valid": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
     "uyd_norm_params_imagenet": (NormParams, []),
     "uyd_norm_params_unit": (NormParams, []),
