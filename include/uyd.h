@@ -373,8 +373,10 @@ int uyd_preprocess_bgra_resize_batch(const uint8_t *d_input, float *d_output, in
                                      int src_width, int src_height, int src_pitch, int dst_width, int dst_height,
                                      uyd_norm_params params, uyd_stream stream);
 
-/* f-1 as SURVEY 8f ranks it: camera bytes feed model.0 DIRECTLY.  The fused stem (uyd_plan_add_stem2 / _pw, which
- * must be the plan's first op) reads the packed BGRA pixels -- bilinearly resampled with the half-pixel rule of
+/* f-1 as SURVEY 8f ranks it: camera bytes feed model.0 DIRECTLY.  The plan's first op must be a stem with a camera
+ * loader: the YAML network's fused stem (uyd_plan_add_stem2 / _pw) or a CUDA-core Conv(3 -> 32, 3x3, stride 2) on the
+ * network input with a 16-byte aligned output slice (model.py's stem at base_channels 32); any other plan returns
+ * UYD_E_UNSUPPORTED before any launch.  The stem reads the packed BGRA pixels -- bilinearly resampled with the half-pixel rule of
  * preprocess_bgra_resize (cuda_preprocess.cu:140-199) when the frame extent differs from the plan's input -- or the
  * NV12 planes (cuda_preprocess.cu:207-253, frame extent == plan input), normalises ((v / 255) - mean) / std on load
  * and never writes a CHW fp32 tensor (4.9 MB written + read back per 640 x 640 frame otherwise).

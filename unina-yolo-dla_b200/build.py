@@ -25,7 +25,7 @@ def _nvcc() -> str:
 
 def build(force: bool = False, verbose: bool = False) -> Path:
     srcs = [CSRC / s for s in SOURCES]
-    deps = srcs + [CSRC / "stem_v2.cuh", CSRC / "c3k_flat.cuh", CSRC / "tc_ptx.cuh", CSRC / "tlbr.cuh", CSRC / "common.cuh", HERE.parent / "include" / "uyd.h"]
+    deps = srcs + [CSRC / "stem_v2.cuh", CSRC / "c3k_flat.cuh", CSRC / "tc_ptx.cuh", CSRC / "tlbr.cuh", CSRC / "camera.cuh", CSRC / "common.cuh", HERE.parent / "include" / "uyd.h"]
     if not force and LIB.exists() and all(d.stat().st_mtime <= LIB.stat().st_mtime for d in deps):
         build_compat(force)
         return LIB

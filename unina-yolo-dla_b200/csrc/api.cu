@@ -6,6 +6,7 @@
 #include <set>
 #include <utility>
 
+#include "camera.cuh"
 #include "common.cuh"
 
 namespace uyd {
@@ -108,10 +109,7 @@ struct StemArgs {
   const uint32_t *wfrag;
   const float *bias;
   int n, ih, iw, oh, ow, out_pitch, u8, pw;
-  int cam, src_w, src_h, src_pitch, uv_pitch;
-  long long frame_stride, uv_frame_stride;
-  const uint8_t *uv;
-  float mean[3], stdv[3];
+  CamFrames f;
 };
 bool stem_fused_supported(int c0, int c1, int ih, int iw, int out_pitch, int out_coff);
 void stem_fused_pack(const float *w0, const float *b0, const float *w1, const float *b1, const float *w2, const float *b2,
@@ -745,7 +743,35 @@ extern "C" int uyd_plan_buffer_ptr(uyd_plan *plan, int id, void **ptr) {
   return UYD_OK;
 }
 
-// x_kind: 1 = NCHW fp32 frames, 2 = NCHW uint8 frames (divided by 255 on load)
+// the frames of a uyd_plan_run_camera call as the stem kernels read them
+static CamFrames cam_frames(const uyd_camera_frames &c) {
+  CamFrames f{};
+  f.cam = c.format; f.src_w = c.width; f.src_h = c.height; f.src_pitch = c.pitch; f.uv_pitch = c.uv_pitch;
+  f.frame_stride = c.frame_stride; f.uv_frame_stride = c.uv_frame_stride; f.uv = c.uv;
+  f.mean[0] = c.norm.mean_r; f.mean[1] = c.norm.mean_g; f.mean[2] = c.norm.mean_b;
+  f.stdv[0] = c.norm.std_r; f.stdv[1] = c.norm.std_g; f.stdv[2] = c.norm.std_b;
+  return f;
+}
+
+// arguments of a CUDA-core OP_CONV (in_buf < 0: the network input x of kind x_kind)
+static ConvArgs direct_conv_args(uyd_plan *plan, const uyd_conv &d, const void *x, int x_kind, int batch, const Op &o) {
+  const Buffer &ob = plan->bufs[d.out_buf];
+  ConvArgs a{};
+  a.n = batch;
+  if (d.in_buf < 0) {
+    a.in = x; a.ih = plan->in_h; a.iw = plan->in_w; a.in_pitch = 0; a.in_nchw_f32 = x_kind;
+  } else {
+    const Buffer &ib = plan->bufs[d.in_buf];
+    a.in = slice_ptr(plan, d.in_buf, d.in_coff); a.ih = ib.h; a.iw = ib.w; a.in_pitch = ib.c;
+  }
+  a.out = slice_ptr(plan, d.out_buf, d.out_coff);
+  a.oh = ob.h; a.ow = ob.w; a.out_pitch = ob.c; a.out_f32 = ob.dtype == UYD_F32;
+  if (d.res_buf >= 0) { a.res = slice_ptr(plan, d.res_buf, d.res_coff); a.res_pitch = plan->bufs[d.res_buf].c; }
+  a.w = o.w_dev; a.bias = o.b_dev; a.cin = d.cin; a.cout = d.cout; a.k = d.k; a.stride = d.stride; a.relu = d.relu;
+  return a;
+}
+
+// x_kind: 1 = NCHW fp32 frames, 2 = NCHW uint8 frames (divided by 255 on load), 3 = plan->cam (uyd_plan_run_camera)
 static int launch_op(uyd_plan *plan, const Op &o, const void *x, int x_kind, int batch, cudaStream_t s, float *y = nullptr) {
   {
     int e = UYD_OK;
@@ -754,21 +780,9 @@ static int launch_op(uyd_plan *plan, const Op &o, const void *x, int x_kind, int
       if (o.use_tc) {
         e = tc_launch(o.tc, 0, batch, plan->ctx->sm_count, s);
       } else {
-        const Buffer &ob = plan->bufs[d.out_buf];
-        ConvArgs a{};
-        a.n = batch;
-        if (d.in_buf < 0) {
-          UYD_REQUIRE(x, UYD_E_ARG, "uyd_plan_run: x is NULL");
-          a.in = x; a.ih = plan->in_h; a.iw = plan->in_w; a.in_pitch = 0; a.in_nchw_f32 = x_kind;
-        } else {
-          const Buffer &ib = plan->bufs[d.in_buf];
-          a.in = slice_ptr(plan, d.in_buf, d.in_coff); a.ih = ib.h; a.iw = ib.w; a.in_pitch = ib.c;
-        }
-        a.out = slice_ptr(plan, d.out_buf, d.out_coff);
-        a.oh = ob.h; a.ow = ob.w; a.out_pitch = ob.c; a.out_f32 = ob.dtype == UYD_F32;
-        if (d.res_buf >= 0) { a.res = slice_ptr(plan, d.res_buf, d.res_coff); a.res_pitch = plan->bufs[d.res_buf].c; }
-        a.w = o.w_dev; a.bias = o.b_dev; a.cin = d.cin; a.cout = d.cout; a.k = d.k; a.stride = d.stride; a.relu = d.relu;
-        e = direct_conv_launch(a, d.depthwise != 0, s);
+        if (d.in_buf < 0) UYD_REQUIRE(x, UYD_E_ARG, "uyd_plan_run: x is NULL");
+        const ConvArgs a = direct_conv_args(plan, d, x, x_kind, batch, o);
+        e = d.in_buf < 0 && x_kind == 3 ? stem_camera_launch(a, cam_frames(plan->cam), s) : direct_conv_launch(a, d.depthwise != 0, s);
       }
     } else if (o.kind == OP_C3K) {
       const Buffer &ib = plan->bufs[o.buf], &ob = plan->bufs[o.out_buf];
@@ -785,13 +799,7 @@ static int launch_op(uyd_plan *plan, const Op &o, const void *x, int x_kind, int
       a.in = x; a.out = (__nv_bfloat16 *)slice_ptr(plan, o.out_buf, o.out_coff);
       a.wfrag = (const uint32_t *)o.w_dev; a.bias = o.b_dev;
       a.n = batch; a.ih = plan->in_h; a.iw = plan->in_w; a.oh = ob.h; a.ow = ob.w; a.out_pitch = ob.c; a.u8 = x_kind == 2; a.pw = o.c;
-      if (x_kind == 3) {
-        const uyd_camera_frames &c = plan->cam;
-        a.cam = c.format; a.src_w = c.width; a.src_h = c.height; a.src_pitch = c.pitch; a.uv_pitch = c.uv_pitch;
-        a.frame_stride = c.frame_stride; a.uv_frame_stride = c.uv_frame_stride; a.uv = c.uv;
-        a.mean[0] = c.norm.mean_r; a.mean[1] = c.norm.mean_g; a.mean[2] = c.norm.mean_b;
-        a.stdv[0] = c.norm.std_r; a.stdv[1] = c.norm.std_g; a.stdv[2] = c.norm.std_b;
-      }
+      if (x_kind == 3) a.f = cam_frames(plan->cam);
       e = stem_fused_launch(a, s);
     } else if (o.kind == OP_CHAIN) {
       UYD_REQUIRE(y || o.chain.out_buf >= 0, UYD_E_ARG, "this plan decodes in its head kernels: run it with uyd_plan_run_decoded");
@@ -879,8 +887,14 @@ extern "C" int uyd_host_free(void *p) {
 
 extern "C" int uyd_plan_run_camera(uyd_plan *plan, const uyd_camera_frames *f, int batch, float *y, uyd_stream stream) {
   UYD_REQUIRE(plan && plan->finalized && f && f->data, UYD_E_ARG, "uyd_plan_run_camera: plan not finalized / NULL frames");
-  UYD_REQUIRE(!plan->ops.empty() && plan->ops[0].kind == OP_STEM2, UYD_E_UNSUPPORTED,
-              "uyd_plan_run_camera: the plan must start with the fused stem (uyd_plan_add_stem2 / _pw)");
+  UYD_REQUIRE(!plan->ops.empty(), UYD_E_UNSUPPORTED, "uyd_plan_run_camera: empty plan");
+  const Op &stem = plan->ops[0];
+  // the YAML network's fused stem, or model.py's Conv 3 -> 32 on the mma stem kernel: the stems with a camera loader
+  const bool conv_stem = stem.kind == OP_CONV && !stem.use_tc && stem.conv.in_buf < 0 && !stem.conv.depthwise &&
+                         stem_camera_supported(direct_conv_args(plan, stem.conv, f->data, 3, 1, stem));
+  UYD_REQUIRE(stem.kind == OP_STEM2 || conv_stem, UYD_E_UNSUPPORTED,
+              "uyd_plan_run_camera: the plan must start with the fused stem (uyd_plan_add_stem2 / _pw) or a Conv(3, 32, 3, 2) on the "
+              "network input");
   UYD_REQUIRE(f->format == UYD_CAM_BGRA || f->format == UYD_CAM_NV12, UYD_E_ARG, "uyd_plan_run_camera: unknown frame format %d", f->format);
   UYD_REQUIRE(f->width > 0 && f->height > 0 && f->norm.std_r != 0.f && f->norm.std_g != 0.f && f->norm.std_b != 0.f, UYD_E_ARG, "uyd_plan_run_camera: bad extent or zero std");
   if (f->format == UYD_CAM_BGRA) {

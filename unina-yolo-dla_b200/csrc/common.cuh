@@ -120,6 +120,11 @@ struct ctx_impl;  // defined in api.cu
 size_t direct_weight_bytes(const uyd_conv &d);
 void direct_pack_weights(const uyd_conv &d, const float *w, void *dst_host);
 int direct_conv_launch(const ConvArgs &a, bool depthwise, cudaStream_t s);
+// Camera frames (camera.cuh) straight into model.py's stem: stem_camera_supported says which stems (Conv 3 -> 32, 3x3,
+// stride 2, on conv_stem_mma_kernel) stem_camera_launch serves; any other returns UYD_E_UNSUPPORTED without a launch.
+struct CamFrames;
+bool stem_camera_supported(const ConvArgs &a);
+int stem_camera_launch(const ConvArgs &a, const CamFrames &f, cudaStream_t s);
 
 size_t direct_weight_bytes_s8(int cin, int cout, int k);
 void direct_pack_weights_s8(int cin, int cout, int k, const int8_t *w, void *dst_host);

@@ -6,6 +6,9 @@
 // Arithmetic follows ConvBlock.forward (model.py:49-50) / Ultralytics Conv with BN folded:
 //   out = [res +] relu(sum_{tap,ci} x * w + bias)
 // One thread = one output pixel x CO_T output channels.
+#include <type_traits>
+
+#include "camera.cuh"
 #include "common.cuh"
 #include "stem_v2.cuh"
 
@@ -336,15 +339,27 @@ __global__ void __launch_bounds__(kStemThreads) conv_stem_tiled_kernel(ConvArgs 
 //   * Rows of m-tile mt are assigned to channels 4 (r & 7) + 2 mt + (r >> 3), so lane (g, t) ends up with channels
 //     4g .. 4g + 3 of pixels 2t and 2t + 1: two 8-byte stores, 64 contiguous bytes per pixel across the warp.
 //   * The loads of tile i + 1 are issued before tile i is computed (tiles strided by the grid).
+//   * TIn = CamIn reads camera frames (camera.cuh) instead of a frame tensor: one 4-pixel vector of a patch row holds all
+//     three channels, so the map runs over (row, vector), 3 raw uint4 per thread in flight (NV12 / BGRA at the model's
+//     extent; converted in stage_cam()).  Resampled BGRA is read and blended in stage_cam(): its 16 taps per vector would not
+//     fit the register budget of two CTAs per SM.
 constexpr int kSmTH = 8, kSmTW = 64, kSmThreads = 256;          // output tile: one row of 64 pixels per warp
 constexpr int kSmIH = 2 * kSmTH + 1, kSmNV = (2 * kSmTW) / 4 + 2;
 constexpr int kSmIP = 152;  // bf16 per patch row (>= 4 kSmNV): row / plane strides of 12 and 20 banks keep the two
                             // combinations one LDS.32 touches in disjoint banks
 static_assert(kSmIP >= 4 * kSmNV && kSmIP % 4 == 0, "patch pitch");
 
+// the camera instantiation's arguments carry the frames
+struct CamConvArgs : ConvArgs {
+  CamFrames f;
+};
+template <typename TIn>
+using StemMmaArgs = typename std::conditional<std::is_same<TIn, CamIn>::value, CamConvArgs, ConvArgs>::type;
+
 template <typename TIn, bool SPLIT>
-__global__ void __launch_bounds__(kSmThreads) conv_stem_mma_kernel(ConvArgs a, int tiles_x, int tiles_y, int total_tiles) {
+__global__ void __launch_bounds__(kSmThreads) conv_stem_mma_kernel(StemMmaArgs<TIn> a, int tiles_x, int tiles_y, int total_tiles) {
   constexpr int NP = SPLIT ? 2 : 1;  // planes: hi (| lo)
+  constexpr bool kCam = std::is_same<TIn, CamIn>::value;
   __shared__ __align__(16) __nv_bfloat16 sx[NP][3][kSmIH][kSmIP];
   __shared__ float sw[27][32];
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, g = lane >> 2, t = lane & 3;
@@ -352,9 +367,9 @@ __global__ void __launch_bounds__(kSmThreads) conv_stem_mma_kernel(ConvArgs a, i
   const bool vec_ok = a.iw % 4 == 0 && (reinterpret_cast<uintptr_t>(a.in) & 15) == 0 && ((long long)a.ih * a.iw * sizeof(TIn)) % 16 == 0;
   // Patch staging: every load of a thread is issued before the first is used (7 x 16 B in flight per thread); the
   // (channel, row, vector) of element i = tid + 256 k advances incrementally (256 = 7 * 34 + 18)
-  constexpr int kIters = (3 * kSmIH * kSmNV + kSmThreads - 1) / kSmThreads;
+  constexpr int kIters = kCam ? (kSmIH * kSmNV + kSmThreads - 1) / kSmThreads : (3 * kSmIH * kSmNV + kSmThreads - 1) / kSmThreads;
   static_assert(kSmThreads / kSmNV < kSmIH, "incremental (c, r, j) update");
-  float4 pv[kIters];
+  typename std::conditional<kCam, uint4, float4>::type pv[kIters];
   auto tile_origin = [&](int tile, int &n, int &oy0, int &ox0) {
     n = tile / (tiles_x * tiles_y);
     const int tr = tile - n * tiles_x * tiles_y;
@@ -364,6 +379,22 @@ __global__ void __launch_bounds__(kSmThreads) conv_stem_mma_kernel(ConvArgs a, i
   auto issue = [&](int tile) {
     int n, oy0, ox0;
     tile_origin(tile, n, oy0, ox0);
+    if constexpr (kCam) {
+      const uint8_t *frame = reinterpret_cast<const uint8_t *>(a.in) + (long long)n * a.f.frame_stride;
+      const uint8_t *uvp = a.f.uv ? a.f.uv + (long long)n * a.f.uv_frame_stride : nullptr;
+      const bool raw = !cam_resampled(a, a.f);
+      int j = tid % kSmNV, r = tid / kSmNV;
+#pragma unroll
+      for (int k = 0; k < kIters; ++k) {
+        const int iy = oy0 * 2 - 1 + r, ix = ox0 * 2 - 4 + 4 * j;
+        uint32_t w[4] = {0u, 0u, 0u, 0u};
+        if (raw && r < kSmIH && iy >= 0 && iy < a.ih && ix >= 0 && ix + 3 < a.iw) cam_load4(a.f, frame, uvp, iy, ix, w);
+        pv[k] = make_uint4(w[0], w[1], w[2], w[3]);
+        j += kSmThreads % kSmNV;
+        r += kSmThreads / kSmNV;
+        if (j >= kSmNV) { j -= kSmNV; ++r; }
+      }
+    } else {
     const TIn *in = reinterpret_cast<const TIn *>(a.in) + (long long)n * 3 * a.ih * a.iw;
     int j = tid % kSmNV, r = tid / kSmNV, c = 0;
 #pragma unroll
@@ -392,29 +423,66 @@ __global__ void __launch_bounds__(kSmThreads) conv_stem_mma_kernel(ConvArgs a, i
       if (j >= kSmNV) { j -= kSmNV; ++r; }
       if (r >= kSmIH) { r -= kSmIH; ++c; }
     }
+    }
   };
   __nv_bfloat16 *sx0 = &sx[0][0][0][0];
   constexpr int kPlane = 3 * kSmIH * kSmIP;  // bf16 elements of the hi plane set
+  // the four values of patch vector (c, r, j) -> hi (| lo) bf16 planes
+  auto put = [&](int c, int r, int j, const float4 &v) {
+    const uint32_t h01 = c3kf::pack_bf16(v.x, v.y), h23 = c3kf::pack_bf16(v.z, v.w);
+    __nv_bfloat16 *d = sx0 + (c * kSmIH + r) * kSmIP + 4 * j;
+    *reinterpret_cast<uint2 *>(d) = make_uint2(h01, h23);
+    if (SPLIT) {  // lo = bf16(x - hi): x = hi + lo up to 2^-17 relative
+      const uint32_t l01 = c3kf::pack_bf16(v.x - c3kf::bf16_lo(h01), v.y - c3kf::bf16_hi(h01));
+      const uint32_t l23 = c3kf::pack_bf16(v.z - c3kf::bf16_lo(h23), v.w - c3kf::bf16_hi(h23));
+      *reinterpret_cast<uint2 *>(d + kPlane) = make_uint2(l01, l23);
+    }
+  };
+  auto stage_cam = [&](int tile) {
+    if constexpr (kCam) {  // zero outside the image (the conv's padding), normalised camera values inside
+      int n, oy0, ox0;
+      tile_origin(tile, n, oy0, ox0);
+      const uint8_t *frame = reinterpret_cast<const uint8_t *>(a.in) + (long long)n * a.f.frame_stride;
+      const CamNorm nm = cam_norm(a.f);
+      const bool resampled = cam_resampled(a, a.f);
+      int j = tid % kSmNV, r = tid / kSmNV;
+#pragma unroll
+      for (int k = 0; k < kIters; ++k) {
+        if (r < kSmIH) {
+          const int iy = oy0 * 2 - 1 + r, ix = ox0 * 2 - 4 + 4 * j;
+          float px[4][3];
+#pragma unroll
+          for (int e = 0; e < 4; ++e) px[e][0] = px[e][1] = px[e][2] = 0.f;
+          if (iy >= 0 && iy < a.ih && ix >= 0 && ix + 3 < a.iw) {
+            if (resampled) {
+              cam_resize4(a, a.f, nm, frame, iy, ix, px);
+            } else {
+              const uint32_t w[4] = {pv[k].x, pv[k].y, pv[k].z, pv[k].w};
+              cam_convert4(a.f, nm, w, px);
+            }
+          }
+#pragma unroll
+          for (int c = 0; c < 3; ++c) put(c, r, j, make_float4(px[0][c], px[1][c], px[2][c], px[3][c]));
+        }
+        j += kSmThreads % kSmNV;
+        r += kSmThreads / kSmNV;
+        if (j >= kSmNV) { j -= kSmNV; ++r; }
+      }
+    }
+  };
   auto stage = [&]() {
+    if constexpr (!kCam) {
     int j = tid % kSmNV, r = tid / kSmNV, c = 0;
 #pragma unroll
     for (int k = 0; k < kIters; ++k) {
       float4 v = pv[k];
       if (sizeof(TIn) == 1) v = make_float4(stemv2::div255(v.x), stemv2::div255(v.y), stemv2::div255(v.z), stemv2::div255(v.w));
-      if (c < 3) {
-        const uint32_t h01 = c3kf::pack_bf16(v.x, v.y), h23 = c3kf::pack_bf16(v.z, v.w);
-        __nv_bfloat16 *d = sx0 + (c * kSmIH + r) * kSmIP + 4 * j;
-        *reinterpret_cast<uint2 *>(d) = make_uint2(h01, h23);
-        if (SPLIT) {  // lo = bf16(x - hi): x = hi + lo up to 2^-17 relative
-          const uint32_t l01 = c3kf::pack_bf16(v.x - c3kf::bf16_lo(h01), v.y - c3kf::bf16_hi(h01));
-          const uint32_t l23 = c3kf::pack_bf16(v.z - c3kf::bf16_lo(h23), v.w - c3kf::bf16_hi(h23));
-          *reinterpret_cast<uint2 *>(d + kPlane) = make_uint2(l01, l23);
-        }
-      }
+      if (c < 3) put(c, r, j, v);
       j += kSmThreads % kSmNV;
       r += kSmThreads / kSmNV;
       if (j >= kSmNV) { j -= kSmNV; ++r; }
       if (r >= kSmIH) { r -= kSmIH; ++c; }
+    }
     }
   };
   int tile = blockIdx.x;
@@ -454,7 +522,8 @@ __global__ void __launch_bounds__(kSmThreads) conv_stem_mma_kernel(ConvArgs a, i
       koff[s][h] = ((combo / 3) * kSmIH + 2 * warp + combo % 3) * kSmIP + 2 + 2 * (t & 1);
     }
   for (; tile < total_tiles; tile += gridDim.x) {
-    stage();
+    if constexpr (kCam) stage_cam(tile);
+    else stage();
     __syncthreads();
     if (tile + (int)gridDim.x < total_tiles) issue(tile + gridDim.x);  // in flight while this tile is computed
     int n, oy0, ox0;
@@ -684,6 +753,28 @@ void direct_pack_weights(const uyd_conv &d, const float *w, void *dst_host) {
         o[((size_t)t * d.cin + ci) * d.cout + co] = __float2bfloat16_rn(w[((size_t)co * d.cin + ci) * taps + t]);
 }
 
+static unsigned stem_mma_grid(const ConvArgs &a, int &tx, int &ty, int &total) {
+  tx = ceil_div(a.ow, kSmTW); ty = ceil_div(a.oh, kSmTH); total = tx * ty * a.n;
+  const int resident = 2 * current_sm_count();  // 256 threads x <= 128 registers: two CTAs per SM
+  return (unsigned)(total < resident ? total : resident);
+}
+
+bool stem_camera_supported(const ConvArgs &a) {
+  return a.cin == 3 && a.cout == 32 && a.k == 3 && a.stride == 2 && !a.out_f32 && !a.res && a.iw % 4 == 0 && a.out_pitch % 8 == 0 &&
+         (reinterpret_cast<uintptr_t>(a.out) & 15) == 0;
+}
+
+int stem_camera_launch(const ConvArgs &a, const CamFrames &f, cudaStream_t s) {
+  UYD_REQUIRE(stem_camera_supported(a), UYD_E_UNSUPPORTED, "camera frames feed only the 3 -> 32 3x3 stride-2 mma stem (16-byte aligned output)");
+  int tx, ty, total;
+  const unsigned mgrid = stem_mma_grid(a, tx, ty, total);
+  CamConvArgs ca;
+  static_cast<ConvArgs &>(ca) = a;
+  ca.f = f;
+  conv_stem_mma_kernel<CamIn, true><<<mgrid, kSmThreads, 0, s>>>(ca, tx, ty, total);
+  return (int)cudaGetLastError();
+}
+
 int direct_conv_launch(const ConvArgs &a, bool depthwise, cudaStream_t s) {
   if (depthwise) {
     UYD_REQUIRE(a.cin % 8 == 0 && a.in_pitch % 8 == 0 && a.out_pitch % 8 == 0 && !a.out_f32 && !a.res &&
@@ -720,9 +811,8 @@ int direct_conv_launch(const ConvArgs &a, bool depthwise, cudaStream_t s) {
     if (a.cin == 3 && (a.cout == 16 || a.cout == 32) && a.k == 3 && a.stride == 2 && a.out_pitch % 8 == 0 &&
         (reinterpret_cast<uintptr_t>(a.out) & 15) == 0) {
       if (a.cout == 32 && a.out_pitch % 4 == 0 && getenv("UYD_STEM_TILED") == nullptr) {
-        const int tx = ceil_div(a.ow, kSmTW), ty = ceil_div(a.oh, kSmTH), total = tx * ty * a.n;
-        const int resident = 2 * current_sm_count();  // 256 threads x ~110 registers: two CTAs per SM
-        const unsigned mgrid = (unsigned)(total < resident ? total : resident);
+        int tx, ty, total;
+        const unsigned mgrid = stem_mma_grid(a, tx, ty, total);
         static const bool split = getenv("UYD_STEM_NO_SPLIT") == nullptr;  // probe: hi plane only (bf16-rounded frame)
         if (split) {
           if (u8) conv_stem_mma_kernel<uint8_t, true><<<mgrid, kSmThreads, 0, s>>>(a, tx, ty, total);

@@ -5,17 +5,21 @@ output ``[(cls[B,nc,H,W], reg[B,4,H,W]) x 3]``; ``predict_batched`` adds the TLB
 class-aware NMS of the reference's post-processing (postprocess.hpp:44-145,
 gpu_postprocess.h:42-80) for the whole batch in one launch and returns ``(det[B,max_det,6], count[B])``
 on the device; ``predict`` returns per-image ``[N,6]`` rows (x1,y1,x2,y2,conf,cls).
+``forward_camera`` / ``predict_camera`` take BGRA or NV12 camera bytes, which the stem reads, normalises
+and resamples itself (no fp32 input tensor).
 """
 from __future__ import annotations
 
 import ctypes as C
 import os
+import types
 
 import torch
 import torch.nn as nn
 
 from . import _lib
 from ._lib import UYD_F32, Detection, check
+from .preprocess import norm_params
 from .plan import NETWORK_INPUT, Plan, Slice, fold_bn
 
 
@@ -188,8 +192,8 @@ class UninaCustomB200(nn.Module):
         cat_f2 = p.buffer(h2, w2, 2 * c2)             # [up(lateral_p2(f3)), p2]
         cat_o3 = p.buffer(h2 // 2, w2 // 2, c2 + c3)  # [down1(f2), f3]
         cat_o4 = p.buffer(h2 // 4, w2 // 4, c3 + c4)  # [down2(o3), p4]
-        x = bb.stem.emit(p, NETWORK_INPUT)
-        x = bb.stage1_conv.emit(p, x)
+        stem = bb.stem.emit(p, NETWORK_INPUT)
+        x = bb.stage1_conv.emit(p, stem)
         p2 = bb.stage1_block.emit(p, x, cat_f2.sub(c2, c2))
         p3 = bb.stage2_c3k2.emit(p, bb.stage2_conv.emit(p, p2), cat_f3.sub(c3, c3))
         p4 = bb.stage3_c3k2.emit(p, bb.stage3_conv.emit(p, p3), cat_o4.sub(c3, c4))
@@ -208,7 +212,7 @@ class UninaCustomB200(nn.Module):
             getattr(self, f"head_p{lvl}").emit(p, f, head, nc)
             heads.append(head)
         p.heads = heads
-        p.feature_slices = {"p2": p2, "p3": p3, "p4": p4, "sppf": ctx, "f2": f2, "o3": o3, "o4": o4}
+        p.feature_slices = {"stem": stem, "p2": p2, "p3": p3, "p4": p4, "sppf": ctx, "f2": f2, "o3": o3, "o4": o4}
         p.finalize()
         # uyd_nms_tlbr reads the head buffers in place: their device pointers and grids, as C arrays, once per plan
         ptrs = []
@@ -237,11 +241,14 @@ class UninaCustomB200(nn.Module):
         """``[(cls, reg)] x 3`` NCHW fp32 (ONNX names p2_cls, p2_reg, ... model.py:382-383)."""
         x = self._prep(x)
         p = self.plan_for(x)
-        B, nc = x.shape[0], self.num_classes
         p.run(x)
+        return self._heads(p, x.shape[0], x.device)
+
+    def _heads(self, p: Plan, B: int, device) -> list:
+        nc = self.num_classes
         outs = []
         for h in p.heads:
-            t = torch.empty(B, nc + 4, h.h, h.w, dtype=torch.float32, device=x.device)
+            t = torch.empty(B, nc + 4, h.h, h.w, dtype=torch.float32, device=device)
             self._export(p, h, t, B)
             outs.append((t[:, :nc], t[:, nc:]))
         return outs
@@ -323,6 +330,107 @@ class UninaCustomB200(nn.Module):
         det = torch.empty(B, max_det, 6, dtype=torch.float32, device=x.device)
         cnt = torch.empty(B, dtype=torch.int32, device=x.device)
         p.run(x)
+        self._nms_tlbr_into(p, B, det, cnt, conf, iou, conformal_q, strict, max_det, max_nms)
+        return det, cnt
+
+    def _camera(self, frames: torch.Tensor, size, norm, uv):
+        """(plan, uyd_camera_frames, batch) for camera bytes on the device; see forward_camera."""
+        if self.training:
+            raise RuntimeError("UninaCustomB200 implements the inference path only: call .eval()")
+        if not (frames.is_cuda and frames.dtype == torch.uint8 and frames.stride(-1) == 1):
+            raise ValueError("frames must be uint8 device bytes with unit stride in the last dimension")
+        nv12 = uv is not None
+        if nv12:
+            if frames.dim() != 3 or not (uv.is_cuda and uv.dtype == torch.uint8 and uv.stride(-1) == 1 and uv.dim() == 3
+                                         and uv.shape[0] == frames.shape[0]):
+                raise ValueError("NV12: frames = Y planes [B,H,W], uv = interleaved UV planes [B,H/2,W], uint8 on the device")
+        elif frames.dim() != 4 or frames.shape[3] != 4:
+            raise ValueError("BGRA frames must be [B,H,W,4]")
+        B, H, W = frames.shape[:3]
+        oh, ow = (H, W) if (nv12 or size is None) else size
+        p = self.plan_for(types.SimpleNamespace(shape=(B, 3, oh, ow), device=frames.device))
+        f = _lib.CameraFrames()
+        f.format = _lib.CAM_NV12 if nv12 else _lib.CAM_BGRA
+        f.width, f.height = W, H
+        f.pitch, f.frame_stride, f.data = frames.stride(1), frames.stride(0), frames.data_ptr()
+        if nv12:
+            f.uv, f.uv_pitch, f.uv_frame_stride = uv.data_ptr(), uv.stride(1), uv.stride(0)
+        f.norm = norm if norm is not None else norm_params()
+        return p, f, B
+
+    @torch.no_grad()
+    def forward_camera(self, frames: torch.Tensor, size=None, norm=None, uv: torch.Tensor | None = None):
+        """Camera bytes straight into the stem (replaces preprocess_bgra_resize / preprocess_nv12 and the CHW fp32
+        tensor, perception_node.cpp:604-612): ``frames`` uint8 device ``[B,H,W,4]`` packed BGRA, resampled bilinearly
+        (half-pixel rule) to ``size=(H',W')`` when given, or -- with ``uv`` ``[B,H/2,W]`` -- the Y planes ``[B,H,W]`` of
+        NV12 frames (BT.601).  Rows may be padded (any pitch; BGRA pitch and frame stride multiples of 4).
+        ``norm``: ``_lib.NormParams``, default ImageNet (``preprocess.norm_params()``), what the node feeds this network
+        (NormParams() in perception_node.cpp); ``UninaYoloB200.forward_camera`` defaults to plain x / 255 instead.
+        Returns ``[(cls, reg)] x 3`` as ``forward`` does.  Only the base_channels-32 stem (Conv 3 -> 32) has a camera
+        loader: other widths raise ``UydError`` (UYD_E_UNSUPPORTED)."""
+        p, f, B = self._camera(frames, size, norm, uv)
+        p.run_camera(f, B)
+        return self._heads(p, B, frames.device)
+
+    def _camera_graph_for(self, frames: torch.Tensor, size, norm, uv, conf, iou, conformal_q, strict, max_det, max_nms):
+        dev = frames.device.index if frames.device.index is not None else torch.cuda.current_device()
+        n = norm if norm is not None else norm_params()
+        key = ("camera", dev, tuple(frames.shape), uv is not None, tuple(uv.shape) if uv is not None else None,
+               tuple(size) if size is not None else None, (n.mean_r, n.mean_g, n.mean_b, n.std_r, n.std_g, n.std_b),
+               float(conf), float(iou), float(conformal_q), bool(strict), int(max_det), int(max_nms))
+        g = self._graphs.get(key)
+        if g is not None:
+            return g
+        fs = torch.empty(frames.shape, dtype=torch.uint8, device=frames.device)   # static, contiguous frame buffers
+        uvs = torch.empty(uv.shape, dtype=torch.uint8, device=frames.device) if uv is not None else None
+        p, f, B = self._camera(fs, size, n, uvs)
+        det = torch.empty(B, max_det, 6, dtype=torch.float32, device=frames.device)
+        cnt = torch.empty(B, dtype=torch.int32, device=frames.device)
+
+        def body():
+            p.run_camera(f, B)
+            self._nms_tlbr_into(p, B, det, cnt, conf, iou, conformal_q, strict, max_det, max_nms)
+
+        fs.copy_(frames)
+        if uv is not None:
+            uvs.copy_(uv)
+        side = torch.cuda.Stream(device=frames.device)
+        side.wait_stream(torch.cuda.current_stream(frames.device))
+        with torch.cuda.stream(side):  # warm-up outside capture (and the plan's argument checks)
+            body()
+        torch.cuda.current_stream(frames.device).wait_stream(side)
+        torch.cuda.synchronize(frames.device)
+        graph = torch.cuda.CUDAGraph()
+        with torch.cuda.graph(graph):
+            body()
+        g = (graph, fs, uvs, det, cnt, p, f)  # the graph reads fs / uvs and writes the plan's buffers, det and cnt
+        self._graphs[key] = g
+        return g
+
+    @torch.no_grad()
+    def predict_camera(self, frames: torch.Tensor, size=None, norm=None, uv=None, conf: float = 0.5, iou: float = 0.45,
+                       conformal_q: float = 0.0, strict: bool = True, max_det: int = 1024, max_nms: int = 0,
+                       graph: bool | None = None):
+        """``forward_camera`` + TLBR decode + NMS, everything on the device: ``(det[B,max_det,6], count[B])`` as
+        ``predict_batched`` returns them, with the same thresholds; frames, ``size``, ``uv`` and ``norm`` (default
+        ImageNet, unlike ``UninaYoloB200.predict_camera``'s plain x / 255) as in ``forward_camera``.  ``graph``
+        (default: batch <= GRAPH_MAX_BATCH) replays the whole step as one CUDA graph that reads static frame buffers;
+        each call copies the frames into them."""
+        if graph is None:
+            graph = frames.shape[0] <= self.GRAPH_MAX_BATCH and os.environ.get("UYD_NO_GRAPH", "0") != "1"
+        if graph:
+            with torch.cuda.device(frames.device):
+                g, fs, uvs, det, cnt, _, _ = self._camera_graph_for(frames, size, norm, uv, conf, iou, conformal_q, strict,
+                                                                    max_det, max_nms)
+                fs.copy_(frames)
+                if uv is not None:
+                    uvs.copy_(uv)
+                g.replay()
+                return det.clone(), cnt.clone()
+        p, f, B = self._camera(frames, size, norm, uv)
+        det = torch.empty(B, max_det, 6, dtype=torch.float32, device=frames.device)
+        cnt = torch.empty(B, dtype=torch.int32, device=frames.device)
+        p.run_camera(f, B)
         self._nms_tlbr_into(p, B, det, cnt, conf, iou, conformal_q, strict, max_det, max_nms)
         return det, cnt
 
