@@ -105,7 +105,11 @@ int uyd_plan_add_stem2_pw(uyd_plan *plan, int out_buf, int out_coff, const float
  * quantised, exact int32 accumulation, y = float(acc) * mult[c] + bias[c] (fp32, separate
  * round-to-nearest multiply and add), optional ReLU.  The output buffer's dtype selects the
  * epilogue: UYD_S8 -> q = clamp(rne(y * out_scale), -127, 127) (the consumer's input quantiser),
- * UYD_F32 / UYD_BF16 -> y.  Bit-exact w.r.t. the integer reference. */
+ * UYD_F32 / UYD_BF16 -> y.  Bit-exact w.r.t. the integer reference.
+ * Tensor-core routes (tcgen05 kind::i8, int8 slices 16-byte aligned, 16-byte output rows): weights resident in shared memory
+ * for cout <= 128 with a power-of-two number of 16-byte lanes per output row; otherwise, when cin % 128 == 0,
+ * cout % 16 == 0, cout <= 256 and there are no partial sums, weights streamed per (channel block, tap)
+ * (uyd_plan_op_info: tc:big-halo / big-pertap / big-flat).  Other convs run on CUDA cores (dp4a). */
 typedef struct uyd_conv_s8 {
   int in_buf, in_coff, out_buf, out_coff;
   int cin, cout, k, stride, relu;

@@ -50,7 +50,8 @@ int tc_prepare(TcConv *tc, const uyd_conv &d, void *in_base, int in_pitch, int i
                int out_pitch, int out_f32, const void *res_base, int res_pitch, void *w_dev, const float *bias_dev,
                int mode_override, int base_offset_mode, int stages_override, int i8 = 0, const float *mult_dev = nullptr,
                float out_scale = 0.f, int out_kind = 0, int halo_pitch = 10);
-bool tc_supported_s8(int cin, int cout, int k, int stride, int in_pitch, int in_coff, int out_pitch, int out_coff, int out_esize);
+bool tc_supported_s8(int cin, int cout, int k, int stride, int in_pitch, int in_coff, int out_pitch, int out_coff, int out_esize,
+                     bool pre);
 size_t tc_weight_bytes_s8(int cin, int cout, int k);
 void tc_pack_weights_s8(int cin, int cout, int k, const int8_t *w, void *dst_host);
 int tc_launch(const TcConv *tc, int n0, int nb, int sm_count, cudaStream_t s);
@@ -363,7 +364,8 @@ extern "C" int uyd_plan_add_conv_s8(uyd_plan *plan, const uyd_conv_s8 *d, const 
   }
   op.out_scale = d->out_scale;
   op.out_kind = ob.dtype == UYD_S8 ? (d->out_round_bf16 ? 3 : 2) : (ob.dtype == UYD_F32 ? 1 : 0);
-  bool tc_ok = !d->depthwise && tc_supported_s8(d->cin, d->cout, d->k, d->stride, ib.c, d->in_coff, ob.c, d->out_coff, (int)ob.elem_bytes());
+  bool tc_ok = !d->depthwise && tc_supported_s8(d->cin, d->cout, d->k, d->stride, ib.c, d->in_coff, ob.c, d->out_coff, (int)ob.elem_bytes(),
+                                             d->pre_buf_p1 != 0);
   if (d->impl == UYD_IMPL_TC) {
     UYD_REQUIRE(tc_ok, UYD_E_UNSUPPORTED, "conv_s8 %d->%d k%d s%d cannot run on the tensor-core path", d->cin, d->cout, d->k, d->stride);
     op.use_tc = true;

@@ -230,9 +230,11 @@ __device__ __forceinline__ void epilogue_chunk_staged(const uint32_t (&raw)[16],
 }
 
 // INT8 path: y = float(acc) * m_c + b_c with separate round-to-nearest multiply and add (the
-// oracle's integer reference, oracle/quant.py), ReLU, then bf16 / fp32 / re-quantised int8.
-__device__ __forceinline__ void epilogue_chunk_i8_staged(const uint32_t (&raw)[16], const float *bias_s, const float *mult_s,
-                                                         int c0, long long pix, const TcParams &p, unsigned char *srow, long long ppix) {
+// oracle's integer reference, oracle/quant.py), ReLU, then bf16 / fp32 / re-quantised int8, written at byte c0 * esize of
+// `srow`: this thread's row of the staging tile (conv_tc_kernel) or its output pixel's row in global memory
+// (conv_tc_big_kernel, whose rows are 16-byte aligned: checked on the host).
+__device__ __forceinline__ void epilogue_chunk_i8(const uint32_t (&raw)[16], const float *bias_s, const float *mult_s,
+                                                  int c0, long long pix, const TcParams &p, unsigned char *srow, long long ppix) {
   float v[16], mv[16], bv[16];
 #pragma unroll
   for (int i = 0; i < 4; ++i) {  // 16-byte broadcast loads of the multiplier / bias vectors
@@ -582,7 +584,7 @@ __global__ void __launch_bounds__(kThreads, 1) conv_tc_kernel(const __grid_const
         }
         if (staged) {
           if (c * 16 < p.cout) {
-            if (I8) epilogue_chunk_i8_staged(cur, bias_s, mult_s, c * 16, pix, p, srow, ppix);
+            if (I8) epilogue_chunk_i8(cur, bias_s, mult_s, c * 16, pix, p, srow, ppix);
             else epilogue_chunk_staged(cur, bias_s, c * 16, pix, p, srow, ppix);
           }
         } else if (pix >= 0 && c * 16 < p.cout) {
@@ -623,15 +625,18 @@ __global__ void __launch_bounds__(kThreads, 1) conv_tc_kernel(const __grid_const
 // 128 / 256 / 512-channel layers of the model.py network, model.py:274-303,308-365).
 //   * a CTA owns a PAIR of M-tiles (a 16 x 16 pixel region, or 256 consecutive pixels of a 1x1 conv) with
 //     two TMEM accumulators of N <= 256 columns: every weight block that crosses L2 -> SMEM feeds 2 x 128 rows;
-//   * weights stream through their own TMA pipeline, one (channel block, tap) block of N x 64 channels per stage;
-//   * activations: HALO (3x3 s1: one [18][18][64] box per channel block, nine tap-shifted descriptors per tile),
-//     PERTAP (3x3 s2: one strided [16][16][64] box per block and tap) or FLAT (1x1: [256][64]).
+//   * weights stream through their own TMA pipeline, one (channel block, tap) block of N x 128 bytes per stage;
+//   * activations: HALO (3x3 s1: one [18][18][128 B] box per channel block, nine tap-shifted descriptors per tile),
+//     PERTAP (3x3 s2: one strided [16][16][128 B] box per block and tap) or FLAT (1x1: [256][128 B]).
+// A 128-byte row is 64 bf16 channels (kind::f16, K = 16 per MMA) or, with I8, 128 int8 channels (kind::i8, K = 32,
+// S32 accumulators, the requant epilogue of the resident int8 kernel): the byte geometry is the same.
 // Warps: 0 = activation TMA, 1 = TMEM allocator + MMA issuer, 2 = weight TMA, 4..11 = two epilogue groups
 // (group g drains M-tile g).  When 4 N <= 512 the accumulator pairs are double-buffered.
 // =================================================================================================
 constexpr int kBigThreads = 128 + 256;
 constexpr int kBigHalo = 18;
 
+template <bool I8>
 __global__ void __launch_bounds__(kBigThreads, 1) conv_tc_big_kernel(const __grid_constant__ CUtensorMap tm_in,
                                                                      const __grid_constant__ CUtensorMap tm_w, const TcParams p) {
   extern __shared__ unsigned char smem_dyn[];
@@ -640,11 +645,12 @@ __global__ void __launch_bounds__(kBigThreads, 1) conv_tc_big_kernel(const __gri
   const uint32_t a_s = base;
   const uint32_t w_s = a_s + (uint32_t)p.stages * p.blk_bytes;
   const uint32_t bar0 = w_s + (uint32_t)p.wstages * p.wblk_bytes;
-  // barrier map: afull[4] aempty[4] wfull[8] wempty[8] tfull[2] tempty[2] | slot | bias[256]
+  // barrier map: afull[4] aempty[4] wfull[8] wempty[8] tfull[2] tempty[2] | slot | bias[256] | mult[256] (I8)
   const uint32_t afull = bar0, aempty = bar0 + 32, wfull = bar0 + 64, wempty = bar0 + 128, tfull = bar0 + 192, tempty = bar0 + 208;
   const uint32_t slot = bar0 + 224;
   uint32_t *slot_ptr = reinterpret_cast<uint32_t *>(smem_dyn + (slot - raw));
   float *bias_s = reinterpret_cast<float *>(smem_dyn + (bar0 + 256u - raw));
+  float *mult_s = reinterpret_cast<float *>(smem_dyn + (bar0 + 1280u - raw));
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int nacc = p.nacc;  // accumulator PAIRS
@@ -657,6 +663,8 @@ __global__ void __launch_bounds__(kBigThreads, 1) conv_tc_big_kernel(const __gri
   }
   griddep_trigger();
   for (int i = threadIdx.x; i < 256; i += kBigThreads) bias_s[i] = i < p.cout ? p.bias[i] : 0.f;
+  if (I8)
+    for (int i = threadIdx.x; i < 256; i += kBigThreads) mult_s[i] = i < p.cout ? p.mult[i] : 0.f;
   if (warp == 1) tmem_alloc(slot, tmem_cols);
   tc_fence_before();
   __syncthreads();
@@ -667,6 +675,7 @@ __global__ void __launch_bounds__(kBigThreads, 1) conv_tc_big_kernel(const __gri
   const int kblocks = p.ncb * p.taps;                                   // weight blocks per pair
   const bool a_per_tap = p.mode == TC_PERTAP;                           // else one A block per channel block
   const long long total = p.total_tiles;                                // pairs of this launch
+  constexpr int cb_elems = I8 ? 128 : 64;                               // channels per 128-byte row
 
   if (warp == 0) {
     // ================= activation TMA =================
@@ -688,12 +697,12 @@ __global__ void __launch_bounds__(kBigThreads, 1) conv_tc_big_kernel(const __gri
           const uint32_t dst = a_s + (uint32_t)stage * p.blk_bytes, fb = afull + 8u * stage;
           mbar_expect_tx(fb, p.tx_bytes);
           if (p.mode == TC_FLAT) {
-            tma_load_2d(dst, &tm_in, fb, j * 64, (int)((long long)p.n0 * p.H * p.W + pair * 256));
+            tma_load_2d(dst, &tm_in, fb, j * cb_elems, (int)((long long)p.n0 * p.H * p.W + pair * 256));
           } else if (p.mode == TC_HALO) {
-            tma_load_4d(dst, &tm_in, fb, j * 64, x0 - 1, y0 - 1, n);
+            tma_load_4d(dst, &tm_in, fb, j * cb_elems, x0 - 1, y0 - 1, n);
           } else {
             const int cb = j / 9, tap = j % 9;
-            tma_load_4d(dst, &tm_in, fb, cb * 64, x0 * p.stride + tap % 3 - 1, y0 * p.stride + tap / 3 - 1, n);
+            tma_load_4d(dst, &tm_in, fb, cb * cb_elems, x0 * p.stride + tap % 3 - 1, y0 * p.stride + tap / 3 - 1, n);
           }
         }
         __syncwarp();
@@ -743,8 +752,10 @@ __global__ void __launch_bounds__(kBigThreads, 1) conv_tc_big_kernel(const __gri
 #pragma unroll
           for (int t = 0; t < 2; ++t) {
 #pragma unroll
-            for (int k = 0; k < 4; ++k)
-              umma_bf16(d0 + (uint32_t)t * p.N, ad + (uint64_t)t * tile_units + 2 * k, wd + 2 * k, p.idesc, (accum | (uint32_t)k) ? 1u : 0u);
+            for (int k = 0; k < 4; ++k) {
+              if (I8) umma_i8(d0 + (uint32_t)t * p.N, ad + (uint64_t)t * tile_units + 2 * k, wd + 2 * k, p.idesc, (accum | (uint32_t)k) ? 1u : 0u);
+              else umma_bf16(d0 + (uint32_t)t * p.N, ad + (uint64_t)t * tile_units + 2 * k, wd + 2 * k, p.idesc, (accum | (uint32_t)k) ? 1u : 0u);
+            }
           }
           umma_commit(wempty + 8u * wstage);
           if (!halo || tap == 8) umma_commit(aempty + 8u * astage);
@@ -764,6 +775,8 @@ __global__ void __launch_bounds__(kBigThreads, 1) conv_tc_big_kernel(const __gri
     const int m = q * 32 + lane;
     const int nchunks = p.N >> 4;
     const unsigned hw = (unsigned)p.H * (unsigned)p.W;
+    unsigned char *out_row = reinterpret_cast<unsigned char *>(p.out);  // I8: rows of out_pitch * esize bytes
+    const long long out_row_pitch = (long long)p.out_pitch * (p.out_kind >= 2 ? 1 : (p.out_kind == 1 ? 4 : 2));
     int it = 0;
     for (long long pair = blockIdx.x; pair < total; pair += gridDim.x, ++it) {
       const int acc = nacc == 2 ? (it & 1) : 0;
@@ -792,7 +805,10 @@ __global__ void __launch_bounds__(kBigThreads, 1) conv_tc_big_kernel(const __gri
           tc_fence_before();
           mbar_arrive(tempty + 8u * acc);
         }
-        if (pix >= 0 && c * 16 < p.cout) epilogue_chunk(cur, bias_s, c * 16, pix, p, -1);
+        if (pix >= 0 && c * 16 < p.cout) {
+          if (I8) epilogue_chunk_i8(cur, bias_s, mult_s, c * 16, pix, p, out_row + pix * out_row_pitch, -1);
+          else epilogue_chunk(cur, bias_s, c * 16, pix, p, -1);
+        }
         if (more) {
           tmem_ld_wait();
 #pragma unroll
@@ -885,17 +901,31 @@ void tc_pack_weights(const uyd_conv &d, const float *w, void *dst_host) {
         }
 }
 
-bool tc_supported_s8(int cin, int cout, int k, int stride, int in_pitch, int in_coff, int out_pitch, int out_coff, int out_esize) {
-  if (!(k == 1 || k == 3) || !(stride == 1 || stride == 2) || (k == 1 && stride != 1)) return false;
-  if (pick_cb_s8(cin) == 0 || cout > 128 || cout < 4) return false;
-  if (in_pitch % 16 || in_coff % 16) return false;
+// int8 on the resident-weight kernel: Cout <= 128, output rows a power-of-two number of 16-byte lanes (staging tile),
+// resident weights + two 128-row stages + one staging group within 227 KB
+static bool tc_resident_fits_s8(int cin, int cout, int k, int out_esize) {
+  if (pick_cb_s8(cin) == 0 || cout > 128) return false;
   const int rb = cout * out_esize;
-  if (rb < 16 || rb > 512 || (rb & (rb - 1)) || (out_pitch * out_esize) % 16 || (out_coff * out_esize) % 16) return false;
+  if (rb < 16 || rb > 512 || (rb & (rb - 1))) return false;
   const int N = (cout + 15) / 16 * 16;
-  // resident weights + two 128-row stages + staging tile must fit
   const size_t need = (((size_t)cin * k * k * N + 1023) & ~(size_t)1023) + 2 * (size_t)128 * pick_cb_s8(cin) + kTailFixed +
                       (size_t)128 * 1 * (N * out_esize + 16) + 1024;  // at least one staging group
   return need <= 227 * 1024;
+}
+
+// int8 on the streamed-weight kernel, taken only where the resident one cannot run: 128-channel blocks,
+// Cout <= 256 in 16-column chunks, direct 16-byte row stores, no partial sums
+static bool tc_big_s8(int cin, int cout, int k, int out_esize, bool pre) {
+  return !tc_resident_fits_s8(cin, cout, k, out_esize) && cin % 128 == 0 && cout % 16 == 0 && cout <= 256 && !pre;
+}
+
+bool tc_supported_s8(int cin, int cout, int k, int stride, int in_pitch, int in_coff, int out_pitch, int out_coff, int out_esize,
+                     bool pre) {
+  if (!(k == 1 || k == 3) || !(stride == 1 || stride == 2) || (k == 1 && stride != 1)) return false;
+  if (pick_cb_s8(cin) == 0 || cout < 4) return false;
+  if (in_pitch % 16 || in_coff % 16) return false;
+  if ((out_pitch * out_esize) % 16 || (out_coff * out_esize) % 16) return false;
+  return tc_resident_fits_s8(cin, cout, k, out_esize) || tc_big_s8(cin, cout, k, out_esize, pre);
 }
 
 size_t tc_weight_bytes_s8(int cin, int cout, int k) { return (size_t)cin * k * k * ((cout + 15) / 16 * 16); }
@@ -912,15 +942,29 @@ void tc_pack_weights_s8(int cin, int cout, int k, const int8_t *w, void *dst_hos
 }
 
 
+// i8: int8 operands (128 channels per row), requant epilogue with mult_dev / out_scale / out_kind as in tc_prepare
 static int tc_prepare_big(TcConv *tc, const uyd_conv &d, void *in_base, int in_pitch, int ih, int iw, int max_batch, void *out_base,
-                          int out_pitch, int out_f32, const void *res_base, int res_pitch, void *w_dev, const float *bias_dev) {
+                          int out_pitch, int out_f32, const void *res_base, int res_pitch, void *w_dev, const float *bias_dev,
+                          int i8 = 0, const float *mult_dev = nullptr, float out_scale = 0.f, int out_kind = 0) {
   TcParams &p = tc->p;
-  UYD_REQUIRE(tc_big_supported(d), UYD_E_UNSUPPORTED, "conv_tc big: cin %% 64, cout %% 16, cout <= 256");
+  const int es = i8 ? 1 : 2, ce = 128 / es;  // bytes per element, channels per 128-byte row
+  UYD_REQUIRE(i8 ? (d.cin % 128 == 0 && d.cout % 16 == 0 && d.cout <= 256 && !d.pre_buf_p1) : tc_big_supported(d), UYD_E_UNSUPPORTED,
+              "conv_tc big: cin %% %d, cout %% 16, cout <= 256, no partial sums", ce);
   UYD_REQUIRE(!res_base || ((res_pitch % 8) == 0 && (reinterpret_cast<uintptr_t>(res_base) & 15) == 0), UYD_E_UNSUPPORTED,
               "conv_tc big: residual slice must be 16-byte aligned");
+  if (i8) {
+    const int esize = out_kind >= 2 ? 1 : (out_kind == 1 ? 4 : 2);
+    UYD_REQUIRE((out_pitch * esize) % 16 == 0 && (reinterpret_cast<uintptr_t>(out_base) & 15) == 0, UYD_E_UNSUPPORTED,
+                "conv_tc big int8: output rows must be 16-byte aligned");
+    p.i8 = 1;
+    p.mult = mult_dev;
+    p.out_scale = out_scale;
+    p.out_kind = out_kind;
+    out_f32 = out_kind == 1;
+  }
   p.big = 1;
   p.cb_bytes = 128;
-  p.ncb = d.cin / 64;
+  p.ncb = d.cin / ce;
   p.taps = d.k * d.k;
   p.stride = d.stride;
   p.N = d.cout;
@@ -929,7 +973,7 @@ static int tc_prepare_big(TcConv *tc, const uyd_conv &d, void *in_base, int in_p
   p.W = d.k == 1 ? iw : (iw + 2 - 3) / d.stride + 1;
   p.mode = d.k == 1 ? TC_FLAT : (d.stride == 1 ? TC_HALO : TC_PERTAP);
   p.layout_type = 2u;
-  p.idesc = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(p.N >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);
+  p.idesc = ((i8 ? 2u : 1u) << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(p.N >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);
   p.pairs_x = ceil_div(p.W, 16);
   p.tiles_y = ceil_div(p.H, 16);
   p.tiles_x = p.pairs_x;
@@ -949,7 +993,7 @@ static int tc_prepare_big(TcConv *tc, const uyd_conv &d, void *in_base, int in_p
   p.blk_bytes = (p.tx_bytes + 1023u) & ~1023u;
   p.wblk_bytes = (uint32_t)p.N * 128u;   // N % 16 == 0 and >= 144: a multiple of 1024 whenever N % 8 == 0
   p.wblk_bytes = (p.wblk_bytes + 1023u) & ~1023u;
-  const size_t tail = 256 + 1024 + 1024;  // barriers + bias
+  const size_t tail = 256 + 1024 + 1024;  // barriers + bias + mult
   const size_t budget = 227 * 1024 - 1024 - tail;
   int stages = p.mode == TC_HALO ? 2 : 3;
   int wstages = (int)((budget - (size_t)stages * p.blk_bytes) / p.wblk_bytes);
@@ -971,31 +1015,31 @@ static int tc_prepare_big(TcConv *tc, const uyd_conv &d, void *in_base, int in_p
   p.bias = bias_dev; p.relu = d.relu;
   tc->w_dev = w_dev;
   const cuuint32_t one4[4] = {1, 1, 1, 1};
-  {  // weights [rows = ncb * taps * N][64 channels]: one box = one (channel block, tap) block
-    const cuuint64_t dims[2] = {64, (cuuint64_t)p.ncb * p.taps * p.N};
+  {  // weights [rows = ncb * taps * N][128 bytes]: one box = one (channel block, tap) block
+    const cuuint64_t dims[2] = {(cuuint64_t)ce, (cuuint64_t)p.ncb * p.taps * p.N};
     const cuuint64_t str[1] = {128};
-    const cuuint32_t box[2] = {64, (cuuint32_t)p.N};
-    if (int e = encode(&tc->tm_w, w_dev, 2, dims, str, box, one4, 128)) return e;
+    const cuuint32_t box[2] = {(cuuint32_t)ce, (cuuint32_t)p.N};
+    if (int e = encode(&tc->tm_w, w_dev, 2, dims, str, box, one4, 128, i8)) return e;
   }
   if (p.mode == TC_FLAT) {
     const cuuint64_t dims[2] = {(cuuint64_t)d.cin, (cuuint64_t)max_batch * ih * iw};
-    const cuuint64_t str[1] = {(cuuint64_t)in_pitch * 2};
-    const cuuint32_t box[2] = {64, 256};
-    if (int e = encode(&tc->tm_in, in_base, 2, dims, str, box, one4, 128)) return e;
+    const cuuint64_t str[1] = {(cuuint64_t)in_pitch * es};
+    const cuuint32_t box[2] = {(cuuint32_t)ce, 256};
+    if (int e = encode(&tc->tm_in, in_base, 2, dims, str, box, one4, 128, i8)) return e;
   } else {
     const cuuint64_t dims[4] = {(cuuint64_t)d.cin, (cuuint64_t)iw, (cuuint64_t)ih, (cuuint64_t)max_batch};
-    const cuuint64_t str[3] = {(cuuint64_t)in_pitch * 2, (cuuint64_t)iw * in_pitch * 2, (cuuint64_t)ih * iw * in_pitch * 2};
+    const cuuint64_t str[3] = {(cuuint64_t)in_pitch * es, (cuuint64_t)iw * in_pitch * es, (cuuint64_t)ih * iw * in_pitch * es};
     if (p.mode == TC_HALO) {
-      const cuuint32_t box[4] = {64, (cuuint32_t)kBigHalo, (cuuint32_t)kBigHalo, 1};
-      if (int e = encode(&tc->tm_in, in_base, 4, dims, str, box, one4, 128)) return e;
+      const cuuint32_t box[4] = {(cuuint32_t)ce, (cuuint32_t)kBigHalo, (cuuint32_t)kBigHalo, 1};
+      if (int e = encode(&tc->tm_in, in_base, 4, dims, str, box, one4, 128, i8)) return e;
     } else {
       const cuuint32_t sd = (cuuint32_t)d.stride;
-      const cuuint32_t box[4] = {64, 16 * sd, 16 * sd, 1};
+      const cuuint32_t box[4] = {(cuuint32_t)ce, 16 * sd, 16 * sd, 1};
       const cuuint32_t estr[4] = {1, sd, sd, 1};
-      if (int e = encode(&tc->tm_in, in_base, 4, dims, str, box, estr, 128)) return e;
+      if (int e = encode(&tc->tm_in, in_base, 4, dims, str, box, estr, 128, i8)) return e;
     }
   }
-  return smem_optin(conv_tc_big_kernel, 227 * 1024);
+  return i8 ? smem_optin(conv_tc_big_kernel<true>, 227 * 1024) : smem_optin(conv_tc_big_kernel<false>, 227 * 1024);
 }
 
 // mode_override: -1 auto, else TC_*.  in_base/out_base/res_base: slice bases of image 0.
@@ -1011,6 +1055,10 @@ int tc_prepare(TcConv *tc, const uyd_conv &d, void *in_base, int in_pitch, int i
     const int Np = (d.cout + 15) / 16 * 16;
     if (!i8 && (d.cout > 128 || (size_t)d.cin * d.k * d.k * Np * 2 > 150 * 1024))
       return tc_prepare_big(tc, d, in_base, in_pitch, ih, iw, max_batch, out_base, out_pitch, out_f32, res_base, res_pitch, w_dev, bias_dev);
+    const int out_esize = out_kind >= 2 ? 1 : (out_kind == 1 ? 4 : 2);
+    if (i8 && tc_big_s8(d.cin, d.cout, d.k, out_esize, d.pre_buf_p1 != 0))
+      return tc_prepare_big(tc, d, in_base, in_pitch, ih, iw, max_batch, out_base, out_pitch, out_f32, res_base, res_pitch, w_dev, bias_dev,
+                            1, mult_dev, out_scale, out_kind);
   }
   const int es = i8 ? 1 : 2;
   const int CB = i8 ? pick_cb_s8(d.cin) : pick_cb(d.cin);
@@ -1175,7 +1223,8 @@ int tc_launch(const TcConv *tc, int n0, int nb, int sm_count, cudaStream_t s) {
     UYD_REQUIRE((long long)(p.n0 + nb) * p.H * p.W < (1ll << 31) && p.total_tiles < (1ll << 24), UYD_E_UNSUPPORTED,
                 "conv_tc big: %d images of %dx%d exceed the kernel's 32-bit pixel index", p.n0 + nb, p.H, p.W);
     const unsigned grid = (unsigned)(p.total_tiles < sm_count ? p.total_tiles : sm_count);
-    UYD_CUDA(launch_pdl(conv_tc_big_kernel, dim3(grid), dim3(kBigThreads), tc->smem, s, tc->tm_in, tc->tm_w, p));
+    if (p.i8) UYD_CUDA(launch_pdl(conv_tc_big_kernel<true>, dim3(grid), dim3(kBigThreads), tc->smem, s, tc->tm_in, tc->tm_w, p));
+    else UYD_CUDA(launch_pdl(conv_tc_big_kernel<false>, dim3(grid), dim3(kBigThreads), tc->smem, s, tc->tm_in, tc->tm_w, p));
     return (int)cudaGetLastError();
   }
   p.total_tiles = p.mode == TC_FLAT ? ((long long)nb * p.H * p.W + 127) / 128 : (long long)nb * p.tiles_x * p.tiles_y;

@@ -6,7 +6,8 @@ class-aware NMS of the reference's post-processing (postprocess.hpp:44-145,
 gpu_postprocess.h:42-80) for the whole batch in one launch and returns ``(det[B,max_det,6], count[B])``
 on the device; ``predict`` returns per-image ``[N,6]`` rows (x1,y1,x2,y2,conf,cls).
 ``forward_camera`` / ``predict_camera`` take BGRA or NV12 camera bytes, which the stem reads, normalises
-and resamples itself (no fp32 input tensor).
+and resamples itself (no fp32 input tensor).  ``calibrate_int8`` / ``set_quantization`` / QAT checkpoints switch the
+convs outside the float layers to INT8 (quant.py), with the YAML network's code (yolo.emit_quant_conv).
 """
 from __future__ import annotations
 
@@ -18,9 +19,11 @@ import torch
 import torch.nn as nn
 
 from . import _lib
+from . import quant as Q
 from ._lib import UYD_F32, Detection, check
 from .preprocess import norm_params
-from .plan import NETWORK_INPUT, Plan, Slice, fold_bn
+from .plan import NETWORK_INPUT, Plan, Slice
+from .yolo import Conv, emit_plain_conv
 
 
 class ConvBlock(nn.Module):
@@ -31,16 +34,11 @@ class ConvBlock(nn.Module):
         self.conv = nn.Conv2d(cin, cout, k, s, k // 2, bias=False)
         self.bn = nn.BatchNorm2d(cout)
         self.act = nn.ReLU(inplace=True)
-        self.k, self.s, self.cout = k, s, cout
+        self.k, self.s, self.g, self.c1, self.c2, self.cout = k, s, 1, cin, cout, cout
 
-    def emit(self, p: Plan, src: Slice, dst: Slice | None = None, res: Slice | None = None) -> Slice:
-        if src.buf < 0:
-            oh, ow = p.in_hw[0] // self.s, p.in_hw[1] // self.s
-        else:
-            oh, ow = (src.h - 1) // self.s + 1, (src.w - 1) // self.s + 1
-        dst = dst or p.buffer(oh, ow, self.cout)
-        w, b = fold_bn(self.conv, self.bn)
-        return p.conv(src, dst, w, b, self.k, self.s, relu=True, res=res)
+    # the YAML network's Conv + BN + ReLU emit: bf16 conv, or in the INT8 graph the quantised conv (with ``feeds``: this
+    # output written as the next quantised conv's int8 input); a conv that reads the network input stays float
+    emit = Conv.emit
 
 
 class Bottleneck(nn.Module):
@@ -53,7 +51,7 @@ class Bottleneck(nn.Module):
         self.add = True
 
     def emit(self, p, src, dst=None):
-        return self.cv2.emit(p, self.cv1.emit(p, src), dst, res=src)
+        return self.cv2.emit(p, self.cv1.emit(p, src, feeds=self.cv2.conv), dst, res=src)
 
 
 class C3k2(nn.Module):
@@ -135,13 +133,17 @@ class DetectionHead(nn.Module):
 
     def emit(self, p, f, head: Slice, nc: int):
         for branch, dst in ((self.cls_branch, head.sub(0, nc)), (self.reg_branch, head.sub(nc, 4))):
-            t = branch[1].emit(p, branch[0].emit(p, f))
-            p.conv(t, dst, branch[2].weight.detach().float().cpu().numpy(), branch[2].bias.detach().float().cpu().numpy(),
-                   1, 1, relu=False)
+            # [0] -> [1] -> [2] each have one consumer: in the INT8 graph each writes the next conv's int8 input
+            t = branch[1].emit(p, branch[0].emit(p, f, feeds=branch[1].conv), feeds=branch[2], feeds_f32=True)
+            emit_plain_conv(p, branch[2], t, dst)
 
 
 class UninaCustomB200(nn.Module):
     STRIDES = (4, 8, 16)
+    # module-name patterns of the convs that stay bf16 in the INT8 graph (QuantSpec.covers: substring match).
+    # PARITY UNPINNED: the reference picks them by pattern (train.py:779); SURVEY 3.5 records "stem" and "head_p2", the
+    # rest of its list is not known.  The stem stays float whatever the patterns say (it reads the network input).
+    FLOAT_LAYERS = ("stem", "head_p2")
 
     def __init__(self, num_classes: int = 4, base_channels: int = 32, lite_p2: bool = False):
         super().__init__()
@@ -150,6 +152,10 @@ class UninaCustomB200(nn.Module):
         self.neck = Neck(self.backbone.out_channels)
         for lvl, c in zip((2, 3, 4), self.neck.out_channels):
             setattr(self, f"head_p{lvl}", DetectionHead(c, num_classes))
+        for name, mod in self.named_modules():
+            if isinstance(mod, nn.Conv2d):
+                mod._uyd_name = name            # the key of the pytorch-quantization ``_amax`` buffers
+        self.quant = None                       # quant.QuantSpec when the INT8 path is active
         self._plans = {}
         self._post = {}
         self._graphs = {}
@@ -172,18 +178,65 @@ class UninaCustomB200(nn.Module):
         return self
 
     def load_state_dict(self, state_dict, strict: bool = True, assign: bool = False):
-        out = super().load_state_dict(state_dict, strict=strict, assign=assign)
+        """Accepts the reference schema (378 entries) plus, for QAT checkpoints, the pytorch-quantization
+        ``<conv>._input_quantizer._amax`` / ``<conv>._weight_quantizer._amax`` buffers, which switch the INT8 path on
+        with the default float layers."""
+        plain, amax = Q.split_state_dict(state_dict)
+        out = super().load_state_dict(plain, strict=strict, assign=assign)
+        if amax:
+            self.set_quantization(amax)
         self.refresh()
         return out
+
+    def set_quantization(self, amax: dict | None, float_layers=FLOAT_LAYERS) -> "UninaCustomB200":
+        """Switches the INT8 path on (``amax``: conv module name -> (input amax, weight amax)) or off (None).
+        Convs whose module name contains one of ``float_layers`` stay bf16 (see FLOAT_LAYERS, PARITY UNPINNED), so do
+        convs without an entry and the stem."""
+        self.quant = Q.QuantSpec(dict(amax), tuple(float_layers)) if amax else None
+        self.refresh()
+        return self
+
+    def quant_state_dict(self) -> dict:
+        """The ``_amax`` buffers of the active quantisation in pytorch-quantization's naming."""
+        return Q.amax_state_dict(self.quant)
+
+    @torch.no_grad()
+    def calibrate_int8(self, frames: torch.Tensor, float_layers=FLOAT_LAYERS, enable: bool = True, method: str = "max",
+                       batch_size: int = 8, percentile: float = 99.99) -> dict:
+        """Static INT8 scales from a calibration set, as ``UninaYoloB200.calibrate_int8`` computes them: ``frames``
+        [N,3,H,W] walked in chunks of ``batch_size`` through the bf16 plan; ``method`` "max" (max |x|), "histogram" /
+        "entropy" (the reference's default), "percentile" or "mse"; weights use the same rule on the host.  Returns
+        ``{conv name: (amax_in, amax_w)}`` for every conv but the stem and, with ``enable``, switches the INT8 path on."""
+        rule = Q.calibration_rule(method)
+        saved, self.quant = self.quant, None
+        try:
+            x_all = self._prep(frames)
+            _, _, H, W = x_all.shape
+            B = min(batch_size, x_all.shape[0])
+            dev = x_all.device.index if x_all.device.index is not None else torch.cuda.current_device()
+            p = self._build_plan(dev, B, H, W, record_inputs=True)
+            names = [n for n, s in p.conv_inputs.items() if s.buf >= 0]
+            a_in = Q.collect_input_amax(p, x_all, B, names, rule, percentile)
+        finally:
+            self.quant = saved
+        convs = {n: m for n, m in self.named_modules() if isinstance(m, nn.Conv2d)}
+        amax = {n: (max(a, 1e-6), Q.weight_amax(convs[n].weight, rule, percentile)) for n, a in zip(names, a_in)}
+        if enable:
+            self.set_quantization(amax, float_layers)
+        return amax
 
     def _apply(self, fn, recurse=True):
         self._plans.clear()
         self._graphs.clear()
         return super()._apply(fn, recurse)
 
-    def _build_plan(self, device, max_batch, H, W) -> Plan:
+    def _build_plan(self, device, max_batch, H, W, record_inputs: bool = False) -> Plan:
+        """``record_inputs`` keeps the input slice of every conv in ``plan.conv_inputs`` (calibration)."""
         p = Plan(device, max_batch)
         p.in_hw = (H, W)
+        p.quant = self.quant
+        if record_inputs:
+            p.conv_inputs = {}
         bb, nk, nc = self.backbone, self.neck, self.num_classes
         c2, c3, c4 = bb.out_channels
         h2, w2 = H // 4, W // 4

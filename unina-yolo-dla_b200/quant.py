@@ -28,13 +28,25 @@ W_SUFFIX = "._weight_quantizer._amax"
 @dataclass
 class QuantSpec:
     amax: dict = field(default_factory=dict)          # conv module name -> (input amax, weight amax)
-    float_layers: tuple = (0, 1, 2)                   # model.{i} kept in floating point (qat.py:700-753)
+    # kept in floating point (qat.py:700-753): an int i names the layer model.{i} (YAML network), a str any conv whose
+    # module name contains it (model.py network, e.g. "stem" or "head_p2")
+    float_layers: tuple = (0, 1, 2)
 
     def covers(self, name: str) -> bool:
         if name not in self.amax:
             return False
         parts = name.split(".")
-        return not (len(parts) > 1 and parts[0] == "model" and parts[1].isdigit() and int(parts[1]) in self.float_layers)
+        layer = int(parts[1]) if len(parts) > 1 and parts[0] == "model" and parts[1].isdigit() else None
+        return not any(f in name if isinstance(f, str) else f == layer for f in self.float_layers)
+
+
+def amax_state_dict(spec: QuantSpec | None) -> dict:
+    """The ``_amax`` buffers of a quantisation in pytorch-quantization's naming."""
+    out = {}
+    for n, (ai, aw) in (spec.amax if spec else {}).items():
+        out[n + IN_SUFFIX] = torch.tensor(ai)
+        out[n + W_SUFFIX] = torch.tensor(aw)
+    return out
 
 
 def scale_of(amax: float) -> np.float32:
@@ -72,6 +84,59 @@ def split_state_dict(sd: dict):
             plain[k] = v
     amax = {n: (amax_in[n], amax_w[n]) for n in amax_in if n in amax_w}
     return plain, amax
+
+
+def calibration_rule(method: str) -> str:
+    """The amax rule of a ``calibrate_int8`` method ("histogram" is the reference's entropy rule)."""
+    rule = {"histogram": "entropy"}.get(method, method)
+    if rule not in ("max", "entropy", "percentile", "mse"):
+        raise ValueError(f"unknown calibration method {method!r}")
+    return rule
+
+
+def collect_input_amax(p, x_all: torch.Tensor, batch: int, names: list, rule: str, percentile: float = 99.99,
+                       per_batch=None) -> list:
+    """Input amax of every conv in ``names`` over the frames ``x_all``, run through the bf16 plan ``p`` in chunks of
+    ``batch``; ``p.conv_inputs`` maps each name to the bf16 slice the conv reads.  Per chunk: one max |x| reduction
+    (uyd_plan_slice_absmax) per input and, unless ``rule`` is "max", one |x| histogram (uyd_plan_slice_histogram);
+    ``per_batch(x, nb)`` runs after them."""
+    from ._lib import UydError
+
+    vmax = [0.0] * len(names)
+    cal = [HistogramCalibrator() for _ in names] if rule != "max" else None
+    for b0 in range(0, x_all.shape[0], batch):
+        x = x_all[b0:b0 + batch].contiguous()
+        nb = x.shape[0]
+        p.run(x)
+        bits = torch.zeros(len(names), dtype=torch.int32, device=x.device)
+        for i, n in enumerate(names):
+            p.slice_absmax(p.conv_inputs[n], nb, bits[i:i + 1])
+        vals = bits.view(torch.float32).cpu().tolist()
+        vmax = [max(a, b) for a, b in zip(vmax, vals)]
+        if cal is not None:
+            nbins = [c.bins_for(v) for c, v in zip(cal, vals)]
+            if max(nbins) > 12288:
+                raise UydError("histogram calibration: a later batch exceeds 6x the first batch's range; "
+                               "put representative frames first")
+            offs = np.concatenate(([0], np.cumsum(nbins)))
+            hist = torch.zeros(int(offs[-1]), dtype=torch.int32, device=x.device)
+            for i, n in enumerate(names):
+                p.slice_histogram(p.conv_inputs[n], nb, 1.0 / cal[i].width, hist[int(offs[i]):int(offs[i + 1])])
+            h = hist.cpu().numpy()
+            for i in range(len(names)):
+                cal[i].add(h[int(offs[i]):int(offs[i + 1])])
+        if per_batch is not None:
+            per_batch(x, nb)
+    return [vmax[i] if rule == "max" else cal[i].compute_amax(rule, percentile) for i in range(len(names))]
+
+
+def weight_amax(w: torch.Tensor, rule: str, percentile: float = 99.99) -> float:
+    """Weight amax on the host with the same rule as the inputs."""
+    if rule == "max":
+        return float(w.detach().abs().max())
+    c = HistogramCalibrator()
+    c.collect_host(w.detach().float().cpu().numpy())
+    return c.compute_amax(rule, percentile)
 
 
 # ------------------------------------------------------------------------------------------------------

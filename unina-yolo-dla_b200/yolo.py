@@ -546,11 +546,7 @@ class UninaYoloB200(nn.Module):
 
     def quant_state_dict(self) -> dict:
         """The ``_amax`` buffers of the active quantisation in pytorch-quantization's naming."""
-        out = {}
-        for n, (ai, aw) in (self.quant.amax if self.quant else {}).items():
-            out[n + Q.IN_SUFFIX] = torch.tensor(ai)
-            out[n + Q.W_SUFFIX] = torch.tensor(aw)
-        return out
+        return Q.amax_state_dict(self.quant)
 
     def _apply(self, fn, recurse=True):
         self._graphs.clear()
@@ -766,11 +762,7 @@ class UninaYoloB200(nn.Module):
           method "percentile" / "mse"      : the other two amax rules of the same calibrator
         Weights use the same method on the host.  Returns ``{conv name: (amax_in, amax_w)}`` and, with ``enable``,
         switches the INT8 path on."""
-        from . import quant as Q
-
-        rule = {"histogram": "entropy"}.get(method, method)
-        if rule not in ("max", "entropy", "percentile", "mse"):
-            raise ValueError(f"unknown calibration method {method!r}")
+        rule = Q.calibration_rule(method)
         saved, self.quant = self.quant, None
         try:
             x_all = self._prep(frames)
@@ -781,30 +773,10 @@ class UninaYoloB200(nn.Module):
             names = [n for n, s in p.conv_inputs.items() if s.buf >= 0]
             det = self.model[-1]
             dfl_name = getattr(det.dfl.conv, "_uyd_name", "")
-            vmax = [0.0] * len(names)
-            cal = [Q.HistogramCalibrator() for _ in names] if rule != "max" else None
             dfl_cal, dfl_max = (Q.HistogramCalibrator() if rule != "max" else None), 0.0
-            for b0 in range(0, x_all.shape[0], B):
-                x = x_all[b0:b0 + B].contiguous()
-                nb = x.shape[0]
-                p.run(x)
-                bits = torch.zeros(len(names), dtype=torch.int32, device=x.device)
-                for i, n in enumerate(names):
-                    p.slice_absmax(p.conv_inputs[n], nb, bits[i:i + 1])
-                vals = bits.view(torch.float32).cpu().tolist()
-                vmax = [max(a, b) for a, b in zip(vmax, vals)]
-                if cal is not None:
-                    nbins = [c.bins_for(v) for c, v in zip(cal, vals)]
-                    if max(nbins) > 12288:
-                        raise _lib.UydError("histogram calibration: a later batch exceeds 6x the first batch's range; "
-                                            "put representative frames first")
-                    offs = np.concatenate(([0], np.cumsum(nbins)))
-                    hist = torch.zeros(int(offs[-1]), dtype=torch.int32, device=x.device)
-                    for i, n in enumerate(names):
-                        p.slice_histogram(p.conv_inputs[n], nb, 1.0 / cal[i].width, hist[int(offs[i]):int(offs[i + 1])])
-                    h = hist.cpu().numpy()
-                    for i in range(len(names)):
-                        cal[i].add(h[int(offs[i]):int(offs[i + 1])])
+
+            def dfl_batch(x, nb):
+                nonlocal dfl_max
                 if dfl_name in p.conv_inputs:  # input of the DFL projection: the softmax probabilities of the box logits
                     for lvl, hd in enumerate(p.heads):
                         t = torch.empty(nb, hd.c, hd.h, hd.w, dtype=torch.float32, device=x.device)
@@ -813,19 +785,10 @@ class UninaYoloB200(nn.Module):
                         dfl_max = max(dfl_max, float(pr.max()))
                         if dfl_cal is not None:
                             dfl_cal.collect_host(pr.cpu().numpy())
+
+            a_in = Q.collect_input_amax(p, x_all, B, names, rule, percentile, per_batch=dfl_batch)
             convs = {n: m for n, m in self.named_modules() if isinstance(m, nn.Conv2d)}
-
-            def w_amax(w):
-                if rule == "max":
-                    return float(w.detach().abs().max())
-                c = Q.HistogramCalibrator()
-                c.collect_host(w.detach().float().cpu().numpy())
-                return c.compute_amax(rule, percentile)
-
-            amax = {}
-            for i, n in enumerate(names):
-                a_in = vmax[i] if rule == "max" else cal[i].compute_amax(rule, percentile)
-                amax[n] = (max(a_in, 1e-6), w_amax(convs[n].weight))
+            amax = {n: (max(a, 1e-6), Q.weight_amax(convs[n].weight, rule, percentile)) for n, a in zip(names, a_in)}
             if dfl_name in p.conv_inputs:
                 amax[dfl_name] = (dfl_max if rule == "max" else dfl_cal.compute_amax(rule, percentile), float(det.reg_max - 1))
         finally:
