@@ -384,8 +384,14 @@ int uyd_preprocess_bgra_resize_batch(const uint8_t *d_input, float *d_output, in
  * preprocess_bgra_resize (cuda_preprocess.cu:140-199) when the frame extent differs from the plan's input -- or the
  * NV12 planes (cuda_preprocess.cu:207-253, frame extent == plan input), normalises ((v / 255) - mean) / std on load
  * and never writes a CHW fp32 tensor (4.9 MB written + read back per 640 x 640 frame otherwise).
+ * UYD_CAM_BGRA_LETTERBOX: packed BGRA of any extent, letterboxed as the Ultralytics predictor does
+ * (LetterBox(center=True, scaleup=True)): the frame is resized, aspect kept, to (new_w, new_h) of
+ * uyd_letterbox_geometry with cv2 4.x's resize(INTER_LINEAR) for uint8, byte for byte, and placed at (top, left) of
+ * the plan's input; every other pixel is byte 114.  Those bytes are normalised as UYD_CAM_BGRA's are, so the stem sees
+ * what the cv2-letterboxed frame as a uint8 tensor gives.  Same layout rules as UYD_CAM_BGRA; a frame whose
+ * letterboxed extent would be empty is UYD_E_ARG.  Boxes go back to frame pixels with uyd_letterbox_boxes.
  * y: decoded output [batch, no, a_total] for plans whose head ops decode in their epilogue, else NULL. */
-enum { UYD_CAM_BGRA = 1, UYD_CAM_NV12 = 2 };
+enum { UYD_CAM_BGRA = 1, UYD_CAM_NV12 = 2, UYD_CAM_BGRA_LETTERBOX = 3 };
 typedef struct uyd_camera_frames {
   int format;                 /* UYD_CAM_*                                                         */
   int width, height;          /* camera frame extent in pixels                                     */
@@ -397,6 +403,23 @@ typedef struct uyd_camera_frames {
   uyd_norm_params norm;
 } uyd_camera_frames;
 int uyd_plan_run_camera(uyd_plan *plan, const uyd_camera_frames *frames, int batch, float *y, uyd_stream stream);
+
+/* Letterbox geometry of a src_w x src_h frame in a dst_w x dst_h model input (Ultralytics LetterBox / scale_boxes):
+ * gain = min(dst_h / src_h, dst_w / src_w) in double, new_w = round(src_w gain), new_h = round(src_h gain),
+ * left = round((dst_w - new_w) / 2 - 0.1), top = round((dst_h - new_h) / 2 - 0.1), rounding half to even as Python's
+ * round does.  UYD_E_ARG for a non-positive extent or a NULL output.  Host only, no device work. */
+int uyd_letterbox_geometry(int src_w, int src_h, int dst_w, int dst_h, int *new_w, int *new_h, int *left, int *top,
+                           double *gain);
+
+/* Boxes of a letterboxed batch back to frame pixels, in place: rows r < count[b] of det [batch, max_det, 6]
+ * (x1, y1, x2, y2, conf, cls; uyd_nms / uyd_nms_tlbr output) get x -= left, y -= top, then x, y times the fp32
+ * reciprocal of (float)gain, then x clamped to [0, src_w] and y to [0, src_h] (NaN kept) -- the float32 result of
+ * Ultralytics' scale_boxes + clip_boxes statements on a CUDA tensor.  Rows past the count and columns 4, 5 are not
+ * touched.  One launch, no host synchronisation (CUDA-graph capturable).  Nothing is launched and UYD_E_ARG is
+ * returned for a NULL pointer, det not aligned to a float, a non-positive batch, max_det or extent, or an empty
+ * letterboxed frame. */
+int uyd_letterbox_boxes(uyd_ctx *ctx, float *det, const int *count, int batch, int max_det, int src_w, int src_h, int dst_w,
+                        int dst_h, uyd_stream stream);
 
 /* Pinned host staging memory for frame batches (cudaHostAlloc).  write_combined != 0: write-combined pages -- the
  * producer (camera driver, decoder) fills them sequentially, the GPU reads them over PCIe without cache snooping;

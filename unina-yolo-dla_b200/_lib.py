@@ -55,7 +55,7 @@ class CameraFrames(C.Structure):
                 ("norm", NormParams)]
 
 
-CAM_BGRA, CAM_NV12 = 1, 2
+CAM_BGRA, CAM_NV12, CAM_BGRA_LETTERBOX = 1, 2, 3
 
 
 class Detection(C.Structure):
@@ -135,6 +135,10 @@ SIGNATURES = {
     "uyd_small_object_metric_update": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_int,
                                                  C.c_double, C.c_double, C.c_double, C.c_void_p, C.c_void_p]),
     "uyd_plan_run_camera": (C.c_int, [C.c_void_p, C.POINTER(CameraFrames), C.c_int, C.c_void_p, C.c_void_p]),
+    "uyd_letterbox_geometry": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_int), C.POINTER(C.c_int),
+                                         C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(C.c_double)]),
+    "uyd_letterbox_boxes": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
+                                      C.c_void_p]),
     "uyd_host_alloc": (C.c_int, [C.c_size_t, C.c_int, C.POINTER(C.c_void_p)]),
     "uyd_host_free": (C.c_int, [C.c_void_p]),
     "uyd_memcpy_d2d": (C.c_int, [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),

@@ -897,9 +897,15 @@ extern "C" int uyd_plan_run_camera(uyd_plan *plan, const uyd_camera_frames *f, i
   UYD_REQUIRE(stem.kind == OP_STEM2 || conv_stem, UYD_E_UNSUPPORTED,
               "uyd_plan_run_camera: the plan must start with the fused stem (uyd_plan_add_stem2 / _pw) or a Conv(3, 32, 3, 2) on the "
               "network input");
-  UYD_REQUIRE(f->format == UYD_CAM_BGRA || f->format == UYD_CAM_NV12, UYD_E_ARG, "uyd_plan_run_camera: unknown frame format %d", f->format);
+  UYD_REQUIRE(f->format == UYD_CAM_BGRA || f->format == UYD_CAM_NV12 || f->format == UYD_CAM_BGRA_LETTERBOX, UYD_E_ARG,
+              "uyd_plan_run_camera: unknown frame format %d", f->format);
   UYD_REQUIRE(f->width > 0 && f->height > 0 && f->norm.std_r != 0.f && f->norm.std_g != 0.f && f->norm.std_b != 0.f, UYD_E_ARG, "uyd_plan_run_camera: bad extent or zero std");
-  if (f->format == UYD_CAM_BGRA) {
+  if (f->format == UYD_CAM_BGRA_LETTERBOX) {
+    const LetterboxGeom g = letterbox_geometry(f->width, f->height, plan->in_w, plan->in_h);
+    UYD_REQUIRE(g.new_w > 0 && g.new_h > 0, UYD_E_ARG, "uyd_plan_run_camera: a %d x %d frame letterboxes to nothing in %d x %d", f->width,
+                f->height, plan->in_w, plan->in_h);
+  }
+  if (f->format != UYD_CAM_NV12) {
     UYD_REQUIRE(f->pitch >= 4 * f->width && f->pitch % 4 == 0 && f->frame_stride % 4 == 0 && (reinterpret_cast<uintptr_t>(f->data) & 3) == 0,
                 UYD_E_ARG, "uyd_plan_run_camera: BGRA pixels must be 4-byte aligned (pitch %% 4 == 0)");
   } else {

@@ -7,7 +7,8 @@
 namespace uyd {
 
 // The frame fields of uyd_camera_frames a stem kernel reads (by value, in the kernel's parameters).
-// cam = 1 packed BGRA (bilinear resize when the frame extent differs from the network input), 2 = NV12;
+// cam = 1 packed BGRA (bilinear resize when the frame extent differs from the network input), 2 = NV12, 3 = packed
+// BGRA letterboxed (CamLetterboxIn instantiations, below);
 // the BGRA pixels / the Y plane are the kernel's input pointer.
 struct CamFrames {
   int cam, src_w, src_h, src_pitch, uv_pitch;
@@ -109,6 +110,96 @@ __device__ __forceinline__ void cam_resize4(const M &m, const CamFrames &f, cons
              wbb * (float)((pbb >> sh) & 0xFF);
     };
     px[j][0] = nm(mix(16), 0); px[j][1] = nm(mix(8), 1); px[j][2] = nm(mix(0), 2);
+  }
+}
+
+// ---- BGRA letterboxed into the model input (f.cam == UYD_CAM_BGRA_LETTERBOX): the Ultralytics predictor's
+// LetterBox(center=True, scaleup=True), i.e. cv2.resize(INTER_LINEAR) of the frame to (new_w, new_h), placed at
+// (top, left), byte 114 around it.  The stem sees the numbers a uint8 tensor of the cv2-letterboxed frame gives.
+struct CamLetterboxIn {};  // TIn tag of the letterboxing instantiations of the stem kernels
+
+// The geometry of a src_w x src_h frame in a dst_w x dst_h model input, shared by the loader, uyd_letterbox_boxes and
+// uyd_letterbox_geometry: r = min(dst_h / src_h, dst_w / src_w), new = round(src * r), pad = round((dst - new) / 2 - 0.1),
+// Python's half-to-even round being nearbyint (1280 x 725 -> new_h = round(362.5) = 362).  gain = r (scale_boxes).
+struct LetterboxGeom {
+  int new_w, new_h, left, top;
+  double gain;
+};
+__host__ __device__ inline LetterboxGeom letterbox_geometry(int src_w, int src_h, int dst_w, int dst_h) {
+  const double r = fmin((double)dst_h / src_h, (double)dst_w / src_w);
+  LetterboxGeom g;
+  g.new_w = (int)nearbyint(src_w * r);
+  g.new_h = (int)nearbyint(src_h * r);
+  g.left = (int)nearbyint((dst_w - g.new_w) / 2.0 - 0.1);
+  g.top = (int)nearbyint((dst_h - g.new_h) / 2.0 - 0.1);
+  g.gain = r;
+  return g;
+}
+
+// the geometry and cv2's source step per axis, scale = 1 / (new / src) in double, once per thread
+struct CamLetterbox {
+  LetterboxGeom g;
+  double scale_x, scale_y;
+};
+template <class M>
+__device__ __forceinline__ CamLetterbox cam_letterbox(const M &m, const CamFrames &f) {
+  CamLetterbox lb;
+  lb.g = letterbox_geometry(f.src_w, f.src_h, m.iw, m.ih);
+  lb.scale_x = 1.0 / ((double)lb.g.new_w / f.src_w);
+  lb.scale_y = 1.0 / ((double)lb.g.new_h / f.src_h);
+  return lb;
+}
+
+// cv2 4.x INTER_LINEAR for uint8, output index d: f = (float)((d + 0.5) scale - 0.5), s = floor(f), f -= s; 11-bit
+// weights rint((1 - f) 2048), rint(f 2048); source indices s, s + 1 clamped to [0, src).  The horizontal pass also
+// zeroes the weight where s falls outside [0, src - 1); the vertical pass does not.  _rn intrinsics: no contraction.
+struct CamTap {
+  int s0, s1, w0, w1;
+};
+__device__ __forceinline__ CamTap cam_lin_tap(int d, double scale, int src, bool clamp_weight) {
+  float f = (float)__dsub_rn(__dmul_rn((double)d + 0.5, scale), 0.5);
+  int s = (int)floorf(f);
+  f = __fsub_rn(f, (float)s);
+  if (clamp_weight) {
+    if (s < 0) { f = 0.f; s = 0; }
+    if (s >= src - 1) { f = 0.f; s = src - 1; }
+  }
+  CamTap t;
+  t.s0 = min(max(s, 0), src - 1);
+  t.s1 = min(max(s + 1, 0), src - 1);
+  t.w0 = __float2int_rn(__fmul_rn(__fsub_rn(1.f, f), 2048.f));
+  t.w1 = __float2int_rn(__fmul_rn(f, 2048.f));
+  return t;
+}
+
+// four horizontally adjacent model-input pixels (iy, ix .. ix + 3): 114 in the pad, else the two passes with cv2's SIMD
+// vertical rounding (((b0 (h0 >> 4)) >> 16) + ((b1 (h1 >> 4)) >> 16) + 2) >> 2.  An exact 2x downscale, where cv2
+// switches to INTER_AREA, gives weights 1024 / 1024 on the 2x2 block here: (a + b + c + d + 2) >> 2 as AREA; a frame
+// already of extent (new_w, new_h) gives weights 2048 / 0: a copy.
+__device__ __forceinline__ void cam_letterbox4(const CamLetterbox &lb, const CamFrames &f, const CamNorm &nm, const uint8_t *frame,
+                                               int iy, int ix, float (&px)[4][3]) {
+  const int y = iy - lb.g.top;
+  const bool row_in = y >= 0 && y < lb.g.new_h;
+  CamTap ty{};
+  if (row_in) ty = cam_lin_tap(y, lb.scale_y, f.src_h, false);
+  const uint8_t *ra = frame + (long long)ty.s0 * f.src_pitch, *rb = frame + (long long)ty.s1 * f.src_pitch;
+#pragma unroll
+  for (int j = 0; j < 4; ++j) {
+    const int x = ix + j - lb.g.left;
+    int v[3] = {114, 114, 114};
+    if (row_in && x >= 0 && x < lb.g.new_w) {
+      const CamTap tx = cam_lin_tap(x, lb.scale_x, f.src_w, true);
+      const uint32_t paa = *reinterpret_cast<const uint32_t *>(ra + 4 * tx.s0), pab = *reinterpret_cast<const uint32_t *>(ra + 4 * tx.s1);
+      const uint32_t pba = *reinterpret_cast<const uint32_t *>(rb + 4 * tx.s0), pbb = *reinterpret_cast<const uint32_t *>(rb + 4 * tx.s1);
+#pragma unroll
+      for (int c = 0; c < 3; ++c) {
+        const int sh = 16 - 8 * c;  // R, G, B = bytes 2, 1, 0
+        const int h0 = (int)((paa >> sh) & 0xFF) * tx.w0 + (int)((pab >> sh) & 0xFF) * tx.w1;
+        const int h1 = (int)((pba >> sh) & 0xFF) * tx.w0 + (int)((pbb >> sh) & 0xFF) * tx.w1;
+        v[c] = (((ty.w0 * (h0 >> 4)) >> 16) + ((ty.w1 * (h1 >> 4)) >> 16) + 2) >> 2;
+      }
+    }
+    px[j][0] = nm((float)v[0], 0); px[j][1] = nm((float)v[1], 1); px[j][2] = nm((float)v[2], 2);
   }
 }
 

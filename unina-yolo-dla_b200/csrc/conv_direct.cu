@@ -342,7 +342,8 @@ __global__ void __launch_bounds__(kStemThreads) conv_stem_tiled_kernel(ConvArgs 
 //   * TIn = CamIn reads camera frames (camera.cuh) instead of a frame tensor: one 4-pixel vector of a patch row holds all
 //     three channels, so the map runs over (row, vector), 3 raw uint4 per thread in flight (NV12 / BGRA at the model's
 //     extent; converted in stage_cam()).  Resampled BGRA is read and blended in stage_cam(): its 16 taps per vector would not
-//     fit the register budget of two CTAs per SM.
+//     fit the register budget of two CTAs per SM.  TIn = CamLetterboxIn (UYD_CAM_BGRA_LETTERBOX) reads and blends its
+//     taps in stage_cam() the same way.
 constexpr int kSmTH = 8, kSmTW = 64, kSmThreads = 256;          // output tile: one row of 64 pixels per warp
 constexpr int kSmIH = 2 * kSmTH + 1, kSmNV = (2 * kSmTW) / 4 + 2;
 constexpr int kSmIP = 152;  // bf16 per patch row (>= 4 kSmNV): row / plane strides of 12 and 20 banks keep the two
@@ -354,12 +355,14 @@ struct CamConvArgs : ConvArgs {
   CamFrames f;
 };
 template <typename TIn>
-using StemMmaArgs = typename std::conditional<std::is_same<TIn, CamIn>::value, CamConvArgs, ConvArgs>::type;
+using StemMmaArgs = typename std::conditional<std::is_same<TIn, CamIn>::value || std::is_same<TIn, CamLetterboxIn>::value, CamConvArgs,
+                                              ConvArgs>::type;
 
 template <typename TIn, bool SPLIT>
 __global__ void __launch_bounds__(kSmThreads) conv_stem_mma_kernel(StemMmaArgs<TIn> a, int tiles_x, int tiles_y, int total_tiles) {
   constexpr int NP = SPLIT ? 2 : 1;  // planes: hi (| lo)
-  constexpr bool kCam = std::is_same<TIn, CamIn>::value;
+  constexpr bool kLetterbox = std::is_same<TIn, CamLetterboxIn>::value;
+  constexpr bool kCam = std::is_same<TIn, CamIn>::value || kLetterbox;
   __shared__ __align__(16) __nv_bfloat16 sx[NP][3][kSmIH][kSmIP];
   __shared__ float sw[27][32];
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, g = lane >> 2, t = lane & 3;
@@ -382,7 +385,7 @@ __global__ void __launch_bounds__(kSmThreads) conv_stem_mma_kernel(StemMmaArgs<T
     if constexpr (kCam) {
       const uint8_t *frame = reinterpret_cast<const uint8_t *>(a.in) + (long long)n * a.f.frame_stride;
       const uint8_t *uvp = a.f.uv ? a.f.uv + (long long)n * a.f.uv_frame_stride : nullptr;
-      const bool raw = !cam_resampled(a, a.f);
+      const bool raw = !kLetterbox && !cam_resampled(a, a.f);
       int j = tid % kSmNV, r = tid / kSmNV;
 #pragma unroll
       for (int k = 0; k < kIters; ++k) {
@@ -445,6 +448,8 @@ __global__ void __launch_bounds__(kSmThreads) conv_stem_mma_kernel(StemMmaArgs<T
       const uint8_t *frame = reinterpret_cast<const uint8_t *>(a.in) + (long long)n * a.f.frame_stride;
       const CamNorm nm = cam_norm(a.f);
       const bool resampled = cam_resampled(a, a.f);
+      CamLetterbox lb;
+      if constexpr (kLetterbox) lb = cam_letterbox(a, a.f);
       int j = tid % kSmNV, r = tid / kSmNV;
 #pragma unroll
       for (int k = 0; k < kIters; ++k) {
@@ -454,7 +459,9 @@ __global__ void __launch_bounds__(kSmThreads) conv_stem_mma_kernel(StemMmaArgs<T
 #pragma unroll
           for (int e = 0; e < 4; ++e) px[e][0] = px[e][1] = px[e][2] = 0.f;
           if (iy >= 0 && iy < a.ih && ix >= 0 && ix + 3 < a.iw) {
-            if (resampled) {
+            if constexpr (kLetterbox) {
+              cam_letterbox4(lb, a.f, nm, frame, iy, ix, px);
+            } else if (resampled) {
               cam_resize4(a, a.f, nm, frame, iy, ix, px);
             } else {
               const uint32_t w[4] = {pv[k].x, pv[k].y, pv[k].z, pv[k].w};
@@ -771,7 +778,8 @@ int stem_camera_launch(const ConvArgs &a, const CamFrames &f, cudaStream_t s) {
   CamConvArgs ca;
   static_cast<ConvArgs &>(ca) = a;
   ca.f = f;
-  conv_stem_mma_kernel<CamIn, true><<<mgrid, kSmThreads, 0, s>>>(ca, tx, ty, total);
+  if (f.cam == UYD_CAM_BGRA_LETTERBOX) conv_stem_mma_kernel<CamLetterboxIn, true><<<mgrid, kSmThreads, 0, s>>>(ca, tx, ty, total);
+  else conv_stem_mma_kernel<CamIn, true><<<mgrid, kSmThreads, 0, s>>>(ca, tx, ty, total);
   return (int)cudaGetLastError();
 }
 

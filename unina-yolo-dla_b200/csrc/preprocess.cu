@@ -7,6 +7,7 @@
 //
 // HBM-bound byte work: the no-resize kernels move 4 pixels per thread (one 16-byte BGRA load, three 16-byte
 // plane stores); the resize kernel gathers four 4-byte pixels per output pixel.
+#include "camera.cuh"  // letterbox_geometry
 #include "common.cuh"
 
 namespace uyd {
@@ -187,5 +188,60 @@ extern "C" int uyd_preprocess_nv12(const uint8_t *d_y_plane, const uint8_t *d_uv
               "uyd_preprocess_nv12: bad arguments");
   dim3 grid(uyd::ceil_div((width + 1) / 2, 256), height);
   uyd::nv12_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(d_y_plane, d_uv_plane, d_output, width, height, y_pitch, uv_pitch, params);
+  return (int)cudaGetLastError();
+}
+
+// ---- letterboxed frames (UYD_CAM_BGRA_LETTERBOX): geometry and boxes back to frame pixels ----
+namespace uyd {
+namespace {
+
+// torch's clamp_(lo, hi) on a CUDA float: NaN stays NaN, else min(max(v, lo), hi)
+__device__ __forceinline__ float clamp_torch(float v, float hi) { return v != v ? v : fminf(fmaxf(v, 0.f), hi); }
+
+// one thread per (image, row); rows past the image's count are left as they are.  The pad is subtracted and the
+// quotient by the gain taken as a product with the fp32 reciprocal, as torch evaluates `boxes[..., :4] /= gain`
+// (a CPU scalar divisor becomes a multiply by 1 / (float)gain); the _rn intrinsics keep the two steps unfused.
+__global__ void __launch_bounds__(256) letterbox_boxes_kernel(float *__restrict__ det, const int *__restrict__ count, int batch,
+                                                              int max_det, float left, float top, float inv_gain, float w0, float h0) {
+  const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= (long long)batch * max_det) return;
+  const int b = (int)(i / max_det), r = (int)(i - (long long)b * max_det);
+  if (r >= count[b]) return;
+  float *d = det + i * 6;
+  d[0] = clamp_torch(__fmul_rn(__fsub_rn(d[0], left), inv_gain), w0);
+  d[1] = clamp_torch(__fmul_rn(__fsub_rn(d[1], top), inv_gain), h0);
+  d[2] = clamp_torch(__fmul_rn(__fsub_rn(d[2], left), inv_gain), w0);
+  d[3] = clamp_torch(__fmul_rn(__fsub_rn(d[3], top), inv_gain), h0);
+}
+
+}  // namespace
+}  // namespace uyd
+
+extern "C" int uyd_letterbox_geometry(int src_w, int src_h, int dst_w, int dst_h, int *new_w, int *new_h, int *left, int *top,
+                                      double *gain) {
+  UYD_REQUIRE(src_w > 0 && src_h > 0 && dst_w > 0 && dst_h > 0 && new_w && new_h && left && top && gain, UYD_E_ARG,
+              "uyd_letterbox_geometry: positive extents and non-NULL outputs required");
+  const uyd::LetterboxGeom g = uyd::letterbox_geometry(src_w, src_h, dst_w, dst_h);
+  *new_w = g.new_w; *new_h = g.new_h; *left = g.left; *top = g.top; *gain = g.gain;
+  return UYD_OK;
+}
+
+extern "C" int uyd_letterbox_boxes(uyd_ctx *ctx, float *det, const int *count, int batch, int max_det, int src_w, int src_h, int dst_w,
+                                   int dst_h, uyd_stream stream) {
+  using namespace uyd;
+  UYD_REQUIRE(det && count && (reinterpret_cast<uintptr_t>(det) & (alignof(float) - 1)) == 0, UYD_E_ARG,
+              "uyd_letterbox_boxes: non-NULL det (float-aligned) and count required");
+  UYD_REQUIRE(batch > 0 && max_det > 0 && src_w > 0 && src_h > 0 && dst_w > 0 && dst_h > 0, UYD_E_ARG,
+              "uyd_letterbox_boxes: batch, max_det and extents must be positive");
+  const LetterboxGeom g = letterbox_geometry(src_w, src_h, dst_w, dst_h);
+  UYD_REQUIRE(g.new_w > 0 && g.new_h > 0, UYD_E_ARG, "uyd_letterbox_boxes: a %d x %d frame letterboxes to nothing in %d x %d", src_w,
+              src_h, dst_w, dst_h);
+  const long long rows = (long long)batch * max_det;
+  UYD_REQUIRE(rows < (1ll << 31), UYD_E_ARG, "uyd_letterbox_boxes: fewer than 2^31 rows required");
+  DeviceGuard guard(ctx_device(ctx));
+  UYD_CUDA(guard.err);
+  const float inv_gain = 1.0f / (float)g.gain;
+  letterbox_boxes_kernel<<<ceil_div((int)rows, 256), 256, 0, (cudaStream_t)stream>>>(det, count, batch, max_det, (float)g.left, (float)g.top,
+                                                                                     inv_gain, (float)src_w, (float)src_h);
   return (int)cudaGetLastError();
 }

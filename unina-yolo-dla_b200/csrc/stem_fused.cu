@@ -82,7 +82,8 @@ __global__ void __launch_bounds__(stemv2::kThreads, PERSIST ? 2 : 3) stem_v2_ker
   // thread (pj, prl): column vector pj of patch rows prl, prl + 15 and (prl < 5) prl + 30 of each channel
   constexpr int kVecPerRow = kInW / 4, kRowLanes = 15;  // 17 vectors per row, 255 loading threads
   static_assert(2 * kRowLanes <= kInH && 3 * kRowLanes >= kInH && kRowLanes * kVecPerRow <= kThreads, "patch load map");
-  constexpr bool kCam = std::is_same<TIn, CamIn>::value;
+  constexpr bool kLetterbox = std::is_same<TIn, CamLetterboxIn>::value;
+  constexpr bool kCam = std::is_same<TIn, CamIn>::value || kLetterbox;
   const TIn *img = reinterpret_cast<const TIn *>(a.in) + (kCam ? 0ll : (long long)n * 3 * a.ih * a.iw);
   asm volatile("" : "+l"(img));  // keep the per-load address arithmetic 32-bit: one IMAD.WIDE.U32 on this base
   const int pj = tid % kVecPerRow, prl = tid / kVecPerRow;
@@ -102,12 +103,17 @@ __global__ void __launch_bounds__(stemv2::kThreads, PERSIST ? 2 : 3) stem_v2_ker
     const uint8_t *frame = reinterpret_cast<const uint8_t *>(a.in) + (long long)n * a.f.frame_stride;
     const uint8_t *uvp = a.f.uv ? a.f.uv + (long long)n * a.f.uv_frame_stride : nullptr;
     const CamNorm nm = cam_norm(a.f);
+    CamLetterbox lb;
+    if constexpr (kLetterbox) lb = cam_letterbox(a, a.f);
 #pragma unroll
     for (int k = 0; k < 3; ++k) {
       float px[4][3];
 #pragma unroll
       for (int j = 0; j < 4; ++j) px[j][0] = px[j][1] = px[j][2] = 0.f;
-      if (ok[k]) cam_row4(a, a.f, nm, frame, uvp, iy0 + prl + kRowLanes * k, ix, px);
+      if (ok[k]) {
+        if constexpr (kLetterbox) cam_letterbox4(lb, a.f, nm, frame, iy0 + prl + kRowLanes * k, ix, px);
+        else cam_row4(a, a.f, nm, frame, uvp, iy0 + prl + kRowLanes * k, ix, px);
+      }
 #pragma unroll
       for (int c = 0; c < 3; ++c)
         pv[c][k] = make_uint4(__float_as_uint(px[0][c]), __float_as_uint(px[1][c]), __float_as_uint(px[2][c]), __float_as_uint(px[3][c]));
@@ -290,6 +296,10 @@ static int stem_v2_launch(const StemArgs &a0, cudaStream_t s) {
   // persistent CTAs pay off once there are several tiles per CTA (batch-1 frames keep one tile per CTA)
   const bool pers = persist && tiles >= 8 * sms;
   using namespace stemv2;
+  if (a.f.cam == UYD_CAM_BGRA_LETTERBOX) {
+    if (a.pw) return pers ? go(stem_v2_kernel<CamLetterboxIn, true, true>, true) : go(stem_v2_kernel<CamLetterboxIn, true, false>, false);
+    return pers ? go(stem_v2_kernel<CamLetterboxIn, false, true>, true) : go(stem_v2_kernel<CamLetterboxIn, false, false>, false);
+  }
   if (a.f.cam) {
     if (a.pw) return pers ? go(stem_v2_kernel<CamIn, true, true>, true) : go(stem_v2_kernel<CamIn, true, false>, false);
     return pers ? go(stem_v2_kernel<CamIn, false, true>, true) : go(stem_v2_kernel<CamIn, false, false>, false);

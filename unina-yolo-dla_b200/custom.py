@@ -21,6 +21,7 @@ import torch.nn as nn
 from . import _lib
 from . import quant as Q
 from ._lib import UYD_F32, Detection, check
+from . import preprocess as P
 from .preprocess import norm_params
 from .plan import NETWORK_INPUT, Plan, Slice
 from .yolo import Conv, emit_plain_conv
@@ -386,13 +387,15 @@ class UninaCustomB200(nn.Module):
         self._nms_tlbr_into(p, B, det, cnt, conf, iou, conformal_q, strict, max_det, max_nms)
         return det, cnt
 
-    def _camera(self, frames: torch.Tensor, size, norm, uv):
+    def _camera(self, frames: torch.Tensor, size, norm, uv, letterbox=False):
         """(plan, uyd_camera_frames, batch) for camera bytes on the device; see forward_camera."""
         if self.training:
             raise RuntimeError("UninaCustomB200 implements the inference path only: call .eval()")
         if not (frames.is_cuda and frames.dtype == torch.uint8 and frames.stride(-1) == 1):
             raise ValueError("frames must be uint8 device bytes with unit stride in the last dimension")
         nv12 = uv is not None
+        if nv12 and letterbox:
+            raise ValueError("letterbox reads packed BGRA frames; NV12 frames are not letterboxed")
         if nv12:
             if frames.dim() != 3 or not (uv.is_cuda and uv.dtype == torch.uint8 and uv.stride(-1) == 1 and uv.dim() == 3
                                          and uv.shape[0] == frames.shape[0]):
@@ -400,10 +403,10 @@ class UninaCustomB200(nn.Module):
         elif frames.dim() != 4 or frames.shape[3] != 4:
             raise ValueError("BGRA frames must be [B,H,W,4]")
         B, H, W = frames.shape[:3]
-        oh, ow = (H, W) if (nv12 or size is None) else size
+        oh, ow = (H, W) if nv12 else P.camera_extent(H, W, size, letterbox)
         p = self.plan_for(types.SimpleNamespace(shape=(B, 3, oh, ow), device=frames.device))
         f = _lib.CameraFrames()
-        f.format = _lib.CAM_NV12 if nv12 else _lib.CAM_BGRA
+        f.format = _lib.CAM_NV12 if nv12 else (_lib.CAM_BGRA_LETTERBOX if letterbox else _lib.CAM_BGRA)
         f.width, f.height = W, H
         f.pitch, f.frame_stride, f.data = frames.stride(1), frames.stride(0), frames.data_ptr()
         if nv12:
@@ -412,37 +415,42 @@ class UninaCustomB200(nn.Module):
         return p, f, B
 
     @torch.no_grad()
-    def forward_camera(self, frames: torch.Tensor, size=None, norm=None, uv: torch.Tensor | None = None):
+    def forward_camera(self, frames: torch.Tensor, size=None, norm=None, uv: torch.Tensor | None = None, letterbox: bool = False):
         """Camera bytes straight into the stem (replaces preprocess_bgra_resize / preprocess_nv12 and the CHW fp32
         tensor, perception_node.cpp:604-612): ``frames`` uint8 device ``[B,H,W,4]`` packed BGRA, resampled bilinearly
         (half-pixel rule) to ``size=(H',W')`` when given, or -- with ``uv`` ``[B,H/2,W]`` -- the Y planes ``[B,H,W]`` of
         NV12 frames (BT.601).  Rows may be padded (any pitch; BGRA pitch and frame stride multiples of 4).
         ``norm``: ``_lib.NormParams``, default ImageNet (``preprocess.norm_params()``), what the node feeds this network
         (NormParams() in perception_node.cpp); ``UninaYoloB200.forward_camera`` defaults to plain x / 255 instead.
+        ``letterbox``: BGRA frames of any extent are letterboxed as the Ultralytics predictor does (aspect-kept cv2
+        INTER_LINEAR resize, grey 114 around it) into ``size``, by default ``preprocess.letterbox_shape(H, W)``.
         Returns ``[(cls, reg)] x 3`` as ``forward`` does.  Only the base_channels-32 stem (Conv 3 -> 32) has a camera
         loader: other widths raise ``UydError`` (UYD_E_UNSUPPORTED)."""
-        p, f, B = self._camera(frames, size, norm, uv)
+        p, f, B = self._camera(frames, size, norm, uv, letterbox)
         p.run_camera(f, B)
         return self._heads(p, B, frames.device)
 
-    def _camera_graph_for(self, frames: torch.Tensor, size, norm, uv, conf, iou, conformal_q, strict, max_det, max_nms):
+    def _camera_graph_for(self, frames: torch.Tensor, size, norm, uv, conf, iou, conformal_q, strict, max_det, max_nms,
+                          letterbox=False):
         dev = frames.device.index if frames.device.index is not None else torch.cuda.current_device()
         n = norm if norm is not None else norm_params()
         key = ("camera", dev, tuple(frames.shape), uv is not None, tuple(uv.shape) if uv is not None else None,
                tuple(size) if size is not None else None, (n.mean_r, n.mean_g, n.mean_b, n.std_r, n.std_g, n.std_b),
-               float(conf), float(iou), float(conformal_q), bool(strict), int(max_det), int(max_nms))
+               float(conf), float(iou), float(conformal_q), bool(strict), int(max_det), int(max_nms), bool(letterbox))
         g = self._graphs.get(key)
         if g is not None:
             return g
         fs = torch.empty(frames.shape, dtype=torch.uint8, device=frames.device)   # static, contiguous frame buffers
         uvs = torch.empty(uv.shape, dtype=torch.uint8, device=frames.device) if uv is not None else None
-        p, f, B = self._camera(fs, size, n, uvs)
+        p, f, B = self._camera(fs, size, n, uvs, letterbox)
         det = torch.empty(B, max_det, 6, dtype=torch.float32, device=frames.device)
         cnt = torch.empty(B, dtype=torch.int32, device=frames.device)
 
         def body():
             p.run_camera(f, B)
             self._nms_tlbr_into(p, B, det, cnt, conf, iou, conformal_q, strict, max_det, max_nms)
+            if letterbox:
+                P.letterbox_boxes(det, cnt, f.height, f.width, *P.camera_extent(f.height, f.width, size, True))
 
         fs.copy_(frames)
         if uv is not None:
@@ -463,28 +471,31 @@ class UninaCustomB200(nn.Module):
     @torch.no_grad()
     def predict_camera(self, frames: torch.Tensor, size=None, norm=None, uv=None, conf: float = 0.5, iou: float = 0.45,
                        conformal_q: float = 0.0, strict: bool = True, max_det: int = 1024, max_nms: int = 0,
-                       graph: bool | None = None):
+                       graph: bool | None = None, letterbox: bool = False):
         """``forward_camera`` + TLBR decode + NMS, everything on the device: ``(det[B,max_det,6], count[B])`` as
         ``predict_batched`` returns them, with the same thresholds; frames, ``size``, ``uv`` and ``norm`` (default
         ImageNet, unlike ``UninaYoloB200.predict_camera``'s plain x / 255) as in ``forward_camera``.  ``graph``
         (default: batch <= GRAPH_MAX_BATCH) replays the whole step as one CUDA graph that reads static frame buffers;
-        each call copies the frames into them."""
+        each call copies the frames into them.  With ``letterbox`` (see ``forward_camera``) the rows are in frame pixels
+        (Ultralytics ``scale_boxes`` + ``clip_boxes``, one launch, inside the graph when there is one)."""
         if graph is None:
             graph = frames.shape[0] <= self.GRAPH_MAX_BATCH and os.environ.get("UYD_NO_GRAPH", "0") != "1"
         if graph:
             with torch.cuda.device(frames.device):
                 g, fs, uvs, det, cnt, _, _ = self._camera_graph_for(frames, size, norm, uv, conf, iou, conformal_q, strict,
-                                                                    max_det, max_nms)
+                                                                    max_det, max_nms, letterbox)
                 fs.copy_(frames)
                 if uv is not None:
                     uvs.copy_(uv)
                 g.replay()
                 return det.clone(), cnt.clone()
-        p, f, B = self._camera(frames, size, norm, uv)
+        p, f, B = self._camera(frames, size, norm, uv, letterbox)
         det = torch.empty(B, max_det, 6, dtype=torch.float32, device=frames.device)
         cnt = torch.empty(B, dtype=torch.int32, device=frames.device)
         p.run_camera(f, B)
         self._nms_tlbr_into(p, B, det, cnt, conf, iou, conformal_q, strict, max_det, max_nms)
+        if letterbox:
+            P.letterbox_boxes(det, cnt, f.height, f.width, *P.camera_extent(f.height, f.width, size, True))
         return det, cnt
 
     @torch.no_grad()

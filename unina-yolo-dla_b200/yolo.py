@@ -24,6 +24,7 @@ import yaml
 
 from . import _lib
 from ._lib import CHAIN_DFL, CHAIN_PW3, CHAIN_STORE, UYD_BF16, UYD_F32, UYD_S8, check
+from . import preprocess as P
 from . import quant as Q
 from .plan import NETWORK_INPUT, Plan, Slice, fold_bn
 
@@ -818,24 +819,29 @@ class UninaYoloB200(nn.Module):
         return y, xs
 
     @torch.no_grad()
-    def forward_camera(self, frames: torch.Tensor, size=None, norm=None, uv: torch.Tensor | None = None) -> torch.Tensor:
+    def forward_camera(self, frames: torch.Tensor, size=None, norm=None, uv: torch.Tensor | None = None,
+                       letterbox: bool = False) -> torch.Tensor:
         """Camera bytes straight into the stem (SURVEY 8f-1; replaces preprocess_bgra_resize / preprocess_nv12 +
         the CHW fp32 tensor, perception_node.cpp:604-612): ``frames`` uint8 device ``[B,H,W,4]`` packed BGRA, resampled
         bilinearly to ``size=(H',W')`` when given, or -- with ``uv`` ``[B,H/2,W]`` -- the Y planes ``[B,H,W]`` of NV12
         frames.  ``norm``: ``_lib.NormParams`` (default: plain x / 255, what the YAML model is fed).
-        Returns the decoded prediction ``y[B,4+nc,A]``."""
+        ``letterbox``: BGRA frames of any extent are letterboxed as the Ultralytics predictor does (aspect-kept
+        cv2 INTER_LINEAR resize, grey 114 around it) into ``size``, by default ``preprocess.letterbox_shape(H, W)``
+        (1280 x 720 -> 384 x 640).  Returns the decoded prediction ``y[B,4+nc,A]`` in model-input pixels."""
         import types
 
         if self.training:
             raise RuntimeError("UninaYoloB200 implements the inference path only: call .eval()")
         assert frames.is_cuda and frames.dtype == torch.uint8 and frames.stride(-1) == 1
         nv12 = uv is not None
+        if nv12 and letterbox:
+            raise ValueError("letterbox reads packed BGRA frames; NV12 frames are not letterboxed")
         B, H, W = frames.shape[:3]
-        oh, ow = (H, W) if (nv12 or size is None) else size
+        oh, ow = (H, W) if nv12 else P.camera_extent(H, W, size, letterbox)
         p = self.plan_for(types.SimpleNamespace(shape=(B, 3, oh, ow), device=frames.device),
                           fused=os.environ.get("UYD_NO_FUSED_DECODE", "0") != "1")
         f = _lib.CameraFrames()
-        f.format = _lib.CAM_NV12 if nv12 else _lib.CAM_BGRA
+        f.format = _lib.CAM_NV12 if nv12 else (_lib.CAM_BGRA_LETTERBOX if letterbox else _lib.CAM_BGRA)
         f.width, f.height = W, H
         f.pitch = frames.stride(1)
         f.frame_stride = frames.stride(0)
@@ -854,9 +860,14 @@ class UninaYoloB200(nn.Module):
 
     @torch.no_grad()
     def predict_camera(self, frames: torch.Tensor, size=None, norm=None, uv=None, conf: float = 0.25, iou: float = 0.7,
-                       max_det: int = 300, max_nms: int = 30000):
-        """``forward_camera`` + NMS: (det[B,max_det,6], count[B]) on the device."""
-        return self.nms(self.forward_camera(frames, size, norm, uv), conf, iou, max_det, max_nms)
+                       max_det: int = 300, max_nms: int = 30000, letterbox: bool = False):
+        """``forward_camera`` + NMS: (det[B,max_det,6], count[B]) on the device.  With ``letterbox`` the rows are in
+        frame pixels (``scale_boxes`` + ``clip_boxes`` of the Ultralytics predictor, one launch)."""
+        det, cnt = self.nms(self.forward_camera(frames, size, norm, uv, letterbox), conf, iou, max_det, max_nms)
+        if letterbox:
+            H, W = frames.shape[1:3]
+            P.letterbox_boxes(det, cnt, H, W, *P.camera_extent(H, W, size, True))
+        return det, cnt
 
     def _nms_workspace(self, dev: int, B: int, A: int, device) -> torch.Tensor:
         need = int(_lib.lib().uyd_nms_workspace_bytes(B, A))
@@ -953,7 +964,7 @@ class UninaYoloB200(nn.Module):
 
     @torch.no_grad()
     def predict_stream(self, batches, conf: float = 0.25, iou: float = 0.7, max_det: int = 300, max_nms: int = 30000,
-                       to_host: bool = True, camera: str | None = None, size=None, norm=None):
+                       to_host: bool = True, camera: str | None = None, size=None, norm=None, letterbox: bool = False):
         """Generator form of ``predict`` (the reference consumes ``YOLO.predict(..., stream=True)``,
         train.py:396-423): ``batches`` yields host frame batches ``[B,3,H,W]`` (uint8 or float, ideally
         pinned).  Batch i+1 is copied host->device on a copy stream while batch i computes, so a
@@ -966,9 +977,13 @@ class UninaYoloB200(nn.Module):
         device tensors are used in place (no staging copy).
         ``camera``: the batches are camera frames read by the stem itself (``forward_camera``): ``"nv12"`` = uint8
         ``[B, 3H/2, W]`` (the Y rows followed by the interleaved UV rows: 1.5 bytes per pixel over PCIe instead of 3),
-        ``"bgra"`` = uint8 ``[B, H, W, 4]`` (resampled to ``size`` when given); ``norm`` as in ``forward_camera``."""
+        ``"bgra"`` = uint8 ``[B, H, W, 4]`` (resampled to ``size`` when given); ``norm`` as in ``forward_camera``.
+        ``letterbox`` (``camera="bgra"`` only): the frames are letterboxed as in ``forward_camera`` and the rows come
+        back in frame pixels."""
         if camera not in (None, "nv12", "bgra"):
             raise ValueError("camera must be None, 'nv12' or 'bgra'")
+        if letterbox and camera != "bgra":
+            raise ValueError("letterbox needs camera='bgra'")
         if not torch.cuda.is_available():
             raise _lib.UydError("no CUDA device: the B200 path has no CPU fallback")
         prm = next(self.parameters())
@@ -1046,7 +1061,7 @@ class UninaYoloB200(nn.Module):
                 hh = xin.shape[1] * 2 // 3
                 y = self.forward_camera(xin[:, :hh], None, norm, xin[:, hh:])
             elif camera == "bgra":
-                y = self.forward_camera(xin, size, norm, None)
+                y = self.forward_camera(xin, size, norm, None, letterbox)
             elif r.n <= self.GRAPH_MAX_BATCH and os.environ.get("UYD_NO_GRAPH", "0") != "1":
                 y = None   # small batches replay the whole step as one CUDA graph
                 r.det, r.cnt = self.predict_batched(xin, conf, iou, max_det, max_nms)
@@ -1059,6 +1074,9 @@ class UninaYoloB200(nn.Module):
                 if y is not None:
                     y.record_stream(post_s)
                     r.det, r.cnt = self.nms(y, conf, iou, max_det, max_nms)
+                    if letterbox:
+                        h0, w0 = xin.shape[1:3]
+                        P.letterbox_boxes(r.det, r.cnt, h0, w0, *P.camera_extent(h0, w0, size, True))
                 if to_host:
                     r.det_h[: r.n].copy_(r.det, non_blocking=True)
                     r.cnt_h[: r.n].copy_(r.cnt, non_blocking=True)
