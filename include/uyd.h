@@ -354,6 +354,33 @@ int uyd_small_object_metric_update(uyd_ctx *ctx, const float *pred, const int *c
                                    const int *gt_count, int gt_max, double size_thr, double iou_thr, double image_size,
                                    unsigned long long *counters, uyd_stream stream);
 
+/* mAP50 / mAP50-95, stage 1: Ultralytics DetectionValidator.match_predictions for every image of the batch, one
+ * launch.  det / count / gt / gt_count as in uyd_eval_update (both in the same pixel space).  For each row i of
+ * image b, record r = b * max_det + i gets:
+ *   tp_mask[r]  bit t set when the row is a TP at IoU threshold iou_thresholds[t] (box_iou >= t, same class; each
+ *               detection keeps its best ground truth, the higher index winning an IoU tie, and each ground truth
+ *               its lowest-index detection);
+ *   sort_key[r] class << 32 | the confidence's bits ordered so that an ascending sort is a descending confidence
+ *               (-0 ranks as +0); rows >= count[b] get INT64_MAX.
+ * n_labels[nc] += the ground truths per class.  A ground truth or a valid row whose class is not an integer in
+ * [0, nc), or a row whose confidence is NaN, is not indexed: it adds 1 to *dropped and its row gets INT64_MAX.
+ * Sorting all records of all calls by key, stably and in (call, image, row) order, gives ap_per_class's order.
+ * Limits: 1 <= n_thresholds <= 16, every threshold > 0 (UYD_E_ARG); nc <= 2^20, gt_max <= 1024 and
+ * max_det <= 1024 (UYD_E_UNSUPPORTED; gt_max is rejected, never clamped).  Nothing is launched on an error. */
+int uyd_eval_match(uyd_ctx *ctx, const float *det, const int *count, int batch, int max_det, const float *gt,
+                   const int *gt_count, int gt_max, int nc, const float *iou_thresholds, int n_thresholds,
+                   unsigned short *tp_mask, long long *sort_key, long long *n_labels, long long *dropped, uyd_stream stream);
+
+/* mAP50 / mAP50-95, stage 2: Ultralytics metrics.ap_per_class per class, one CTA per class, bit-exact fp64.
+ * sorted_key [n_records] ascending (uyd_eval_match keys after a stable sort), order [n_records] the record index of
+ * each sorted key into tp_mask, n_labels [nc] from uyd_eval_match.  Writes ap [nc, n_thresholds] (compute_ap, the
+ * 101-point interpolation), p_curve / r_curve [nc, 1000] (precision / recall at confidences np.linspace(0, 1, 1000),
+ * threshold 0).  A class without records or without labels gets zeros.  Limits: n_records > 0, 1 <= n_thresholds
+ * <= 16 (UYD_E_ARG); nc <= 2^20 (UYD_E_UNSUPPORTED). */
+int uyd_eval_ap(uyd_ctx *ctx, const long long *sorted_key, const long long *order, const unsigned short *tp_mask,
+                long long n_records, const long long *n_labels, int nc, int n_thresholds, double *ap, double *p_curve,
+                double *r_curve, uyd_stream stream);
+
 /* ------------------------------------------------------------------------------------
  * Camera-frame pre-processing in front of the plan (drop-in for cuda_preprocess.h:62-84; kernels
  * cuda_preprocess.cu:99-253): BGRA / NV12 bytes -> RGB, (x / 255 - mean) / std, planar CHW fp32.

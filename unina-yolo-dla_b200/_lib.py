@@ -134,6 +134,10 @@ SIGNATURES = {
                                   C.c_float, C.c_float, C.c_void_p, C.c_void_p, C.c_void_p]),
     "uyd_small_object_metric_update": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_int,
                                                  C.c_double, C.c_double, C.c_double, C.c_void_p, C.c_void_p]),
+    "uyd_eval_match": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_int,
+                                 C.POINTER(C.c_float), C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "uyd_eval_ap": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_longlong, C.c_void_p, C.c_int, C.c_int,
+                              C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "uyd_plan_run_camera": (C.c_int, [C.c_void_p, C.POINTER(CameraFrames), C.c_int, C.c_void_p, C.c_void_p]),
     "uyd_letterbox_geometry": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_int), C.POINTER(C.c_int),
                                          C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(C.c_double)]),

@@ -1,26 +1,44 @@
 """Batched evaluation consumer of the detections (reference: UninaValidator trainer.py:196-286, the
-small-object metrics; calibrate_conformal_prediction train.py:299-520, the conformal quantile).  Everything
+small-object metrics; calibrate_conformal_prediction train.py:299-520, the conformal quantile; with ``nc`` set,
+the box metrics of Ultralytics ``model.val``: precision, recall, mAP50, mAP50-95 and fitness).  Everything
 stays on the GPU; with several ranks the detections are gathered first (dp.gather_detections, the only
-collective of the path) or the counters / scores are reduced at the end (``reduce``)."""
+collective of the path) or the counters / scores / records are reduced at the end (``reduce``)."""
 from __future__ import annotations
 
 import ctypes as C
 
+import numpy as np
 import torch
 
 from . import _lib
 from ._lib import check
 
 
+# Ultralytics DetectionValidator.iouv and DetMetrics.keys
+MAP_IOUV = torch.linspace(0.5, 0.95, 10)
+MAP_KEYS = ("metrics/precision(B)", "metrics/recall(B)", "metrics/mAP50(B)", "metrics/mAP50-95(B)")
+_PAD_KEY = torch.iinfo(torch.int64).max   # the key of a padding row: sorts behind every class
+
+
 class DetectionEvaluator:
-    def __init__(self, size_threshold: float = 15.0, small_iou: float = 0.45, match_iou: float = 0.5, device=None):
+    """``nc`` (opt-in) also collects, per ``update``, the records ``map_metrics`` turns into mAP50 / mAP50-95 for
+    classes 0 .. nc - 1; with ``nc=None`` nothing of that runs."""
+
+    def __init__(self, size_threshold: float = 15.0, small_iou: float = 0.45, match_iou: float = 0.5, device=None, nc=None):
         self.size_threshold, self.small_iou, self.match_iou = float(size_threshold), float(small_iou), float(match_iou)
         self.device = torch.device(device if device is not None else f"cuda:{torch.cuda.current_device()}")
+        self.nc = None if nc is None else int(nc)
+        if self.nc is not None and self.nc <= 0:
+            raise ValueError("nc must be positive")
         self.reset()
 
     def reset(self) -> None:
         self.counters = torch.zeros(3, dtype=torch.int64, device=self.device)   # small-object TP, FP, FN
         self._scores = []
+        if self.nc is not None:
+            self._n_labels = torch.zeros(self.nc, dtype=torch.int64, device=self.device)
+            self._dropped = torch.zeros(1, dtype=torch.int64, device=self.device)
+            self._keys, self._masks = [], []   # per update: sort keys [B * max_det] int64, TP masks (uint16 bits in int16)
 
     @torch.no_grad()
     def update(self, det: torch.Tensor, cnt: torch.Tensor, gt: torch.Tensor, gt_cnt: torch.Tensor) -> None:
@@ -38,24 +56,74 @@ class DetectionEvaluator:
                                          C.c_void_p(scores.data_ptr()), C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)),
               "uyd_eval_update")
         self._scores.append(scores)
+        if self.nc is not None:
+            keys = torch.empty(B * max_det, dtype=torch.int64, device=det.device)
+            masks = torch.empty(B * max_det, dtype=torch.int16, device=det.device)
+            thr = (C.c_float * len(MAP_IOUV))(*MAP_IOUV.tolist())
+            check(_lib.lib().uyd_eval_match(_lib.context(dev), C.c_void_p(det.data_ptr()), C.c_void_p(cnt.data_ptr()), B, max_det,
+                                            C.c_void_p(gt.data_ptr()), C.c_void_p(gt_cnt.data_ptr()), gt.shape[1], self.nc, thr,
+                                            len(MAP_IOUV), C.c_void_p(masks.data_ptr()), C.c_void_p(keys.data_ptr()),
+                                            C.c_void_p(self._n_labels.data_ptr()), C.c_void_p(self._dropped.data_ptr()),
+                                            C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)),
+                  "uyd_eval_match")
+            self._keys.append(keys)
+            self._masks.append(masks)
 
     def reduce(self, group=None) -> None:
-        """Sums the counters and concatenates the scores over the ranks (when every rank evaluated its own shard)."""
+        """Sums the counters and concatenates the scores over the ranks (when every rank evaluated its own shard).
+        With ``nc`` set it also sums the label counts and gathers the mAP records in rank order, so with contiguous
+        ``dp.shard_bounds`` shards equal confidences rank as in one process."""
         import torch.distributed as dist
 
         if not (dist.is_available() and dist.is_initialized()) or dist.get_world_size(group) == 1:
             return
         dist.all_reduce(self.counters, group=group)
         s = torch.cat([t.flatten() for t in self._scores]) if self._scores else torch.empty(0, device=self.device)
-        n = torch.tensor([s.numel()], device=self.device)
-        sizes = [torch.zeros_like(n) for _ in range(dist.get_world_size(group))]
-        dist.all_gather(sizes, n, group=group)
-        m = int(max(int(x) for x in sizes))
-        pad = torch.full((m,), -1.0, device=self.device)
-        pad[: s.numel()] = s
-        out = [torch.empty_like(pad) for _ in sizes]
-        dist.all_gather(out, pad, group=group)
-        self._scores = [torch.cat(out)]
+        self._scores = [_all_gather_padded(s, -1.0, group)]
+        if self.nc is not None:
+            dist.all_reduce(self._n_labels, group=group)
+            dist.all_reduce(self._dropped, group=group)
+            keys = torch.cat(self._keys) if self._keys else torch.empty(0, dtype=torch.int64, device=self.device)
+            masks = torch.cat(self._masks) if self._masks else torch.empty(0, dtype=torch.int16, device=self.device)
+            self._keys = [_all_gather_padded(keys, _PAD_KEY, group)]
+            self._masks = [_all_gather_padded(masks.int(), 0, group).short()]   # int32 on the wire: gloo has no int16
+
+    @torch.no_grad()
+    def map_metrics(self) -> dict:
+        """The box metrics of Ultralytics ``model.val`` over everything ``update`` saw: the results dict (keys
+        metrics/precision(B), metrics/recall(B), metrics/mAP50(B), metrics/mAP50-95(B), fitness) plus the per-class
+        ``ap50``, ``ap`` (mean over IoU 0.5:0.95) and ``ap_class_index`` arrays, classes with labels only.
+        One stable device sort of the records, one ap_per_class launch, then numpy on [classes, 1000] arrays."""
+        return map_results(*self._ap_per_class())
+
+    def _ap_per_class(self):
+        """(ap [nc, 10], p_curve [nc, 1000], r_curve [nc, 1000]) as fp64 numpy, or Nones without any record, and
+        the label counts [nc]."""
+        if self.nc is None:
+            raise RuntimeError("map_metrics needs DetectionEvaluator(nc=...)")
+        dropped = int(self._dropped)
+        if dropped:
+            raise ValueError(f"{dropped} ground truths / detections had a class outside [0, {self.nc}) or a NaN confidence")
+        T = len(MAP_IOUV)
+        n_labels = self._n_labels.cpu().numpy()
+        keys = torch.cat(self._keys) if self._keys else torch.empty(0, dtype=torch.int64, device=self.device)
+        ap = p_curve = r_curve = None
+        if keys.numel():
+            masks = torch.cat(self._masks)
+            # The one step left to torch: a stable device sort of all records by (class, confidence descending); the
+            # stable order keeps (update call, image, row) among equal keys.  libuyd ships no radix sort of its own.
+            skeys, order = torch.sort(keys, stable=True)
+            ap = torch.empty(self.nc, T, dtype=torch.float64, device=self.device)
+            p_curve = torch.empty(self.nc, 1000, dtype=torch.float64, device=self.device)
+            r_curve = torch.empty(self.nc, 1000, dtype=torch.float64, device=self.device)
+            dev = self.device.index if self.device.index is not None else torch.cuda.current_device()
+            check(_lib.lib().uyd_eval_ap(_lib.context(dev), C.c_void_p(skeys.data_ptr()), C.c_void_p(order.data_ptr()),
+                                         C.c_void_p(masks.data_ptr()), keys.numel(), C.c_void_p(self._n_labels.data_ptr()),
+                                         self.nc, T, C.c_void_p(ap.data_ptr()), C.c_void_p(p_curve.data_ptr()),
+                                         C.c_void_p(r_curve.data_ptr()), C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)),
+                  "uyd_eval_ap")
+            ap, p_curve, r_curve = ap.cpu().numpy(), p_curve.cpu().numpy(), r_curve.cpu().numpy()
+        return ap, p_curve, r_curve, n_labels
 
     def small_object_metrics(self) -> dict:
         """trainer.py:267-285 (the 1e-7 guards included)."""
@@ -85,6 +153,53 @@ class DetectionEvaluator:
         return {"alpha": alpha, "coverage_target": 1 - alpha, "q_hat": q_hat, "dilation_factor": q_hat,
                 "num_calibration_samples": int(srt.numel()), "mean_nonconformity": float(s.mean()),
                 "std_nonconformity": float(s.std(unbiased=False))}
+
+
+def _all_gather_padded(x: torch.Tensor, pad_value, group) -> torch.Tensor:
+    """Concatenation in rank order of every rank's 1-D ``x``, each padded to the longest with ``pad_value``."""
+    import torch.distributed as dist
+
+    n = torch.tensor([x.numel()], device=x.device)
+    sizes = [torch.zeros_like(n) for _ in range(dist.get_world_size(group))]
+    dist.all_gather(sizes, n, group=group)
+    m = int(max(int(v) for v in sizes))
+    pad = torch.full((m,), pad_value, dtype=x.dtype, device=x.device)
+    pad[: x.numel()] = x
+    out = [torch.empty_like(pad) for _ in sizes]
+    dist.all_gather(out, pad, group=group)
+    return torch.cat(out)
+
+
+def _smooth(y: np.ndarray, f: float = 0.05) -> np.ndarray:
+    """Ultralytics utils.metrics.smooth: box filter of odd width round(len * 2f) // 2 + 1, edges padded."""
+    nf = round(len(y) * f * 2) // 2 + 1
+    p = np.ones(nf // 2)
+    yp = np.concatenate((p * y[0], y, p * y[-1]), 0)
+    return np.convolve(yp, np.ones(nf) / nf, mode="valid")
+
+
+def map_results(ap, p_curve, r_curve, n_labels, eps: float = 1e-16) -> dict:
+    """The host tail of Ultralytics ap_per_class and DetMetrics.results_dict over the per-class outputs of
+    ``uyd_eval_ap`` (ap [nc, 10], p_curve / r_curve [nc, 1000] fp64, n_labels [nc]): keep the classes with labels,
+    F1 = 2pr / (p + r + eps), the argmax of its smoothed class mean picks one confidence for P and R.  Like
+    DetectionValidator.get_stats, when no prediction is a TP at any threshold (then every ap is 0; any TP makes its
+    class's ap positive) nothing is reported and every metric is 0."""
+    sel = np.flatnonzero(np.asarray(n_labels) > 0)
+    if ap is None or not (ap[sel] > 0).any():
+        p = r = np.zeros(0)
+        all_ap = np.zeros((0, len(MAP_IOUV)))
+        sel = np.zeros(0, dtype=int)
+    else:
+        all_ap, pc, rc = ap[sel], p_curve[sel], r_curve[sel]
+        f1 = 2 * pc * rc / (pc + rc + eps)
+        i = _smooth(f1.mean(0), 0.1).argmax()
+        p, r = pc[:, i], rc[:, i]
+    mean = [p.mean() if len(p) else 0.0, r.mean() if len(r) else 0.0, all_ap[:, 0].mean() if len(all_ap) else 0.0,
+            all_ap.mean() if len(all_ap) else 0.0]
+    fitness = (np.nan_to_num(np.array(mean)) * [0.0, 0.0, 0.1, 0.9]).sum()
+    out = dict(zip(MAP_KEYS + ("fitness",), mean + [fitness]))
+    out.update(ap50=all_ap[:, 0].copy(), ap=all_ap.mean(1), ap_class_index=sel.astype(int))
+    return out
 
 
 class SmallObjectMetric:
