@@ -20,6 +20,8 @@
  *   uyd_nms                 <- Ultralytics non_max_suppression + torchvision.ops.nms
  *                              (train.py:396-405) and run_gpu_nms + copy_valid_detections_to_host
  *                              (gpu_postprocess.h:70-78)
+ *   uyd_nms_ex              <- the same with multi_label / classes (DetectionValidator.postprocess,
+ *                              YOLO.predict(classes=))
  *   uyd_nms_tlbr            <- decode_yolo_head x3 + run_gpu_nms of a whole batch in one launch
  *                              (perception_node.cpp:581-689)
  */
@@ -282,6 +284,26 @@ int uyd_nms(uyd_ctx *ctx, const float *y, int batch, int nc, int anchors, float 
             double iou_thr, int max_nms, int max_det, float max_wh, void *workspace,
             size_t workspace_bytes, float *out_det, int *out_idx, int *out_count,
             uyd_stream stream);
+
+/* The non_max_suppression options of Ultralytics that uyd_nms does not take. */
+typedef struct uyd_nms_options {
+  int multi_label;           /* 0: best class per anchor (uyd_nms); 1: every (anchor, class) with score > conf_thr */
+  int num_filter_classes;    /* entries of filter_classes (host array); ignored when filter_classes is NULL */
+  const int *filter_classes; /* NULL: all classes; non-NULL: keep only these ids (ids outside [0, nc) match nothing,
+                                0 entries keep nothing) */
+} uyd_nms_options;
+
+/* uyd_nms with options (opt == NULL is uyd_nms itself; no workspace is needed).
+ *   multi_label (with nc > 1): every (anchor, class) pair with score > conf_thr is a candidate, ranked by score
+ *     descending, then anchor, then class ascending (the row-major order of Ultralytics' torch.where under a stable
+ *     sort); the row's conf is that class's score and out_idx its anchor.  max_nms then counts pairs.
+ *   filter_classes: applied to the best class of an anchor (an anchor whose best class is not listed is dropped; it
+ *     does not fall back to another class), or to each pair under multi_label -- before the max_nms truncation.
+ * Class-agnostic NMS is max_wh = 0.  UYD_E_ARG, with nothing launched, for num_filter_classes < 0 or > 0 with a
+ * NULL filter_classes, besides the errors of uyd_nms.  No host synchronisation (CUDA-graph capturable). */
+int uyd_nms_ex(uyd_ctx *ctx, const float *y, int batch, int nc, int anchors, float conf_thr, double iou_thr,
+               int max_nms, int max_det, float max_wh, const uyd_nms_options *opt, float *out_det, int *out_idx,
+               int *out_count, uyd_stream stream);
 
 /* Greedy class-aware NMS over uyd_detection records (postprocess.hpp:44-67 semantics:
  * confidence-descending, same class, IoU > thr; ties broken by cell_idx ascending, or by

@@ -58,6 +58,11 @@ class CameraFrames(C.Structure):
 CAM_BGRA, CAM_NV12, CAM_BGRA_LETTERBOX = 1, 2, 3
 
 
+class NmsOptions(C.Structure):
+    """uyd_nms_options (include/uyd.h)."""
+    _fields_ = [("multi_label", C.c_int), ("num_filter_classes", C.c_int), ("filter_classes", C.POINTER(C.c_int))]
+
+
 class Detection(C.Structure):
     """Layout-identical to the reference GpuDetection (gpu_postprocess.h:27-33)."""
     _fields_ = [("x1", C.c_float), ("y1", C.c_float), ("x2", C.c_float), ("y2", C.c_float),
@@ -113,6 +118,8 @@ SIGNATURES = {
     "uyd_nms_workspace_bytes": (C.c_size_t, [C.c_int, C.c_int]),
     "uyd_nms": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_float, C.c_double, C.c_int, C.c_int,
                           C.c_float, C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "uyd_nms_ex": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_float, C.c_double, C.c_int, C.c_int,
+                             C.c_float, C.POINTER(NmsOptions), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "uyd_nms_detections_workspace_bytes": (C.c_size_t, [C.c_int]),
     "uyd_nms_detections": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_float, C.c_void_p,
                                      C.c_size_t, C.c_void_p, C.c_void_p, C.c_void_p]),

@@ -45,8 +45,9 @@ __device__ __forceinline__ bool suppresses(const float4 &a, float aa, int ca, co
 }
 
 // =================================================================================================
-// Fused per-image NMS (the default path of uyd_nms): ONE launch, one 1024-thread CTA per image.
-//   1. scan   : best class / score per anchor, conf filter, 64-bit key (score code | anchor | class); the keys
+// Fused per-image NMS (uyd_nms / uyd_nms_ex): ONE launch, one 1024-thread CTA per image.
+//   1. scan   : best class / score per anchor (MULTI: every (anchor, class) pair), conf filter, class filter
+//               (FILTER: after the best class is chosen, or per pair), 64-bit key (score code | anchor | class); the keys
 //               of the current slab are captured in shared memory.  A slab is a key range holding at most
 //               kFCap candidates: normally the whole image (<= kFCap candidates: one pass over the scores);
 //               dense scenes are cut into consecutive ranges with a 2048-bin histogram of the key space
@@ -91,67 +92,111 @@ struct FusedSmem {
   int warp_cnt[kFThreads / 32];
   unsigned long long kmin, kmax, cut;
   int count, kept, alive;
+  unsigned cmask[8];  // FILTER: bit c set = class c is kept
 };
 
-__global__ void __launch_bounds__(kFThreads, 1) nms_image_kernel(const float *__restrict__ y, int nc, int A, float conf_thr,
-                                                                 float iou_thr, int max_nms, int max_det, float max_wh, int pos,
-                                                                 float *__restrict__ out_det, int *__restrict__ out_idx,
-                                                                 int *__restrict__ out_count) {
+struct ClassMask {  // the class filter of uyd_nms_options as 256 bits (nc <= 256)
+  unsigned w[8];
+};
+
+// MULTI: one candidate per (anchor, class) with score > conf_thr (Ultralytics multi_label=True); otherwise one per anchor,
+// its best class.  FILTER: only the classes set in cmask become candidates.  The default call is <false, false>.
+template <bool MULTI, bool FILTER>
+__device__ __forceinline__ void nms_image(const float *__restrict__ y, int nc, int A, float conf_thr, float iou_thr, int max_nms,
+                                          int max_det, float max_wh, int pos, float *__restrict__ out_det,
+                                          int *__restrict__ out_idx, int *__restrict__ out_count, const ClassMask &cmask) {
   extern __shared__ __align__(16) unsigned char fused_raw[];
   FusedSmem &S = *reinterpret_cast<FusedSmem *>(fused_raw);
   const int b = blockIdx.x, tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
   const float *yb = y + (long long)b * (4 + nc) * A;
-  if (tid == 0) S.kept = 0;
+  if (tid == 0) {
+    S.kept = 0;
+    if (FILTER) {
+#pragma unroll
+      for (int i = 0; i < 8; ++i) S.cmask[i] = cmask.w[i];
+    }
+  }
   unsigned long long lo = 0ull;   // keys below lo have been consumed
   int processed = 0;
   __syncthreads();
+  auto kept_class = [&](int c) { return !FILTER || ((S.cmask[c >> 5] >> (c & 31)) & 1u) != 0u; };
 
   // mode 0: count keys in [lo, hi), track min / max, capture the first kFCap;  mode 1: histogram over (key - kmin) >> shift
   auto scan = [&](unsigned long long hi, int mode, int shift) {
     constexpr int U = 4;  // anchors per thread and round: U independent loads in flight per class plane
     unsigned long long mn = ~0ull, mx = 0ull;  // per-thread key range, reduced once after the loop
-    for (int a0 = 0; a0 < A; a0 += U * kFThreads) {
-      float best[U];
-      int bj[U];
-#pragma unroll
-      for (int u = 0; u < U; ++u) {
-        const int a = a0 + u * kFThreads + tid;
-        best[u] = a < A ? yb[4ll * A + a] : -INFINITY;
-        bj[u] = 0;
+    // every lane of the warp calls this for each of its keys (in = false for none)
+    auto offer = [&](bool in, unsigned long long key) {
+      if (mode == 0) {
+        const unsigned bal = __ballot_sync(0xffffffffu, in);
+        if (bal) {
+          int base = 0;
+          if (lane == 0) base = atomicAdd(&S.count, __popc(bal));
+          base = __shfl_sync(0xffffffffu, base, 0);
+          if (in) {
+            const int slot = base + __popc(bal & ((1u << lane) - 1));
+            if (slot < kFCap) S.keys[slot] = key;
+            mn = key < mn ? key : mn;
+            mx = key > mx ? key : mx;
+          }
+        }
+      } else if (in) {
+        atomicAdd(&S.hist[(unsigned)((key - S.kmin) >> shift)], 1u);
       }
-      for (int c = 1; c < nc; ++c) {
-        const float *pc = yb + (4ll + c) * A;
+    };
+    for (int a0 = 0; a0 < A; a0 += U * kFThreads) {
+      if constexpr (MULTI) {
+        // class planes in order; a plane the filter drops is not read at all (c is uniform across the CTA)
+        for (int c = 0; c < nc; ++c) {
+          if (!kept_class(c)) continue;
+          const float *pc = yb + (4ll + c) * A;
+          float v[U];
+#pragma unroll
+          for (int u = 0; u < U; ++u) {
+            const int a = a0 + u * kFThreads + tid;
+            v[u] = a < A ? pc[a] : -INFINITY;
+          }
+#pragma unroll
+          for (int u = 0; u < U; ++u) {
+            const int a = a0 + u * kFThreads + tid;
+            bool in = false;
+            unsigned long long key = 0ull;
+            if (a < A && v[u] > conf_thr) {
+              key = fused_key(v[u], c, a, pos != 0);
+              in = key >= lo && key < hi;
+            }
+            offer(in, key);
+          }
+        }
+      } else {
+        float best[U];
+        int bj[U];
 #pragma unroll
         for (int u = 0; u < U; ++u) {
           const int a = a0 + u * kFThreads + tid;
-          const float v = a < A ? pc[a] : -INFINITY;
-          if (v > best[u]) { best[u] = v; bj[u] = c; }   // first maximum wins
+          best[u] = a < A ? yb[4ll * A + a] : -INFINITY;
+          bj[u] = 0;
         }
-      }
+        for (int c = 1; c < nc; ++c) {
+          const float *pc = yb + (4ll + c) * A;
 #pragma unroll
-      for (int u = 0; u < U; ++u) {
-        const int a = a0 + u * kFThreads + tid;
-        bool in = false;
-        unsigned long long key = 0ull;
-        if (a < A && best[u] > conf_thr) {
-          key = fused_key(best[u], bj[u], a, pos != 0);
-          in = key >= lo && key < hi;
-        }
-        if (mode == 0) {
-          const unsigned bal = __ballot_sync(0xffffffffu, in);
-          if (bal) {
-            int base = 0;
-            if (lane == 0) base = atomicAdd(&S.count, __popc(bal));
-            base = __shfl_sync(0xffffffffu, base, 0);
-            if (in) {
-              const int slot = base + __popc(bal & ((1u << lane) - 1));
-              if (slot < kFCap) S.keys[slot] = key;
-              mn = key < mn ? key : mn;
-              mx = key > mx ? key : mx;
-            }
+          for (int u = 0; u < U; ++u) {
+            const int a = a0 + u * kFThreads + tid;
+            const float v = a < A ? pc[a] : -INFINITY;
+            if (v > best[u]) { best[u] = v; bj[u] = c; }   // first maximum wins
           }
-        } else if (in) {
-          atomicAdd(&S.hist[(unsigned)((key - S.kmin) >> shift)], 1u);
+        }
+#pragma unroll
+        for (int u = 0; u < U; ++u) {
+          const int a = a0 + u * kFThreads + tid;
+          bool in = false;
+          unsigned long long key = 0ull;
+          // the filter applies to the chosen class: an anchor whose best class is dropped does not fall back to another
+          if (a < A && best[u] > conf_thr && kept_class(bj[u])) {
+            key = fused_key(best[u], bj[u], a, pos != 0);
+            in = key >= lo && key < hi;
+          }
+          offer(in, key);
         }
       }
     }
@@ -324,6 +369,20 @@ __global__ void __launch_bounds__(kFThreads, 1) nms_image_kernel(const float *__
     if (out_idx) out_idx[(long long)b * max_det + k] = k < kept ? S.kanchor[k] : -1;
   }
   if (tid == 0) out_count[b] = kept;
+}
+
+// One entry point for the four instances (bit 1 of mode: MULTI, bit 0: FILTER), so the library keeps a single NMS
+// kernel symbol; the mode is uniform over the launch and each CTA runs exactly one inlined instance.
+__global__ void __launch_bounds__(kFThreads, 1) nms_image_kernel(const float *__restrict__ y, int nc, int A, float conf_thr,
+                                                                 float iou_thr, int max_nms, int max_det, float max_wh, int pos,
+                                                                 float *__restrict__ out_det, int *__restrict__ out_idx,
+                                                                 int *__restrict__ out_count, int mode, ClassMask cmask) {
+  switch (mode) {
+    case 0: nms_image<false, false>(y, nc, A, conf_thr, iou_thr, max_nms, max_det, max_wh, pos, out_det, out_idx, out_count, cmask); break;
+    case 1: nms_image<false, true>(y, nc, A, conf_thr, iou_thr, max_nms, max_det, max_wh, pos, out_det, out_idx, out_count, cmask); break;
+    case 2: nms_image<true, false>(y, nc, A, conf_thr, iou_thr, max_nms, max_det, max_wh, pos, out_det, out_idx, out_count, cmask); break;
+    default: nms_image<true, true>(y, nc, A, conf_thr, iou_thr, max_nms, max_det, max_wh, pos, out_det, out_idx, out_count, cmask); break;
+  }
 }
 
 // =================================================================================================
@@ -687,24 +746,43 @@ extern "C" size_t uyd_nms_workspace_bytes(int batch, int anchors) {  // kept for
   return (batch > 0 && anchors > 0) ? 256 : 0;
 }
 
-extern "C" int uyd_nms(uyd_ctx *ctx, const float *y, int batch, int nc, int anchors, float conf_thr, double iou_thr,
-                       int max_nms, int max_det, float max_wh, void *workspace, size_t workspace_bytes, float *out_det,
-                       int *out_idx, int *out_count, uyd_stream stream) {
+extern "C" int uyd_nms_ex(uyd_ctx *ctx, const float *y, int batch, int nc, int anchors, float conf_thr, double iou_thr,
+                          int max_nms, int max_det, float max_wh, const uyd_nms_options *opt, float *out_det, int *out_idx,
+                          int *out_count, uyd_stream stream) {
   using namespace uyd;
-  (void)workspace; (void)workspace_bytes;
   UYD_REQUIRE(y && out_det && out_count && batch > 0 && nc > 0 && anchors > 0, UYD_E_ARG, "uyd_nms: bad arguments");
+  UYD_REQUIRE(!opt || (opt->num_filter_classes >= 0 && (opt->num_filter_classes == 0 || opt->filter_classes)), UYD_E_ARG,
+              "uyd_nms_ex: num_filter_classes must be >= 0, and > 0 only with a filter_classes array");
   DeviceGuard guard(ctx_device(ctx));
   UYD_REQUIRE(nc <= 256 && anchors < (1 << kAnchorBits), UYD_E_UNSUPPORTED, "uyd_nms: nc <= 256 and anchors < 4M per image");
   UYD_REQUIRE(max_det > 0 && max_det <= kMaxDetCap, UYD_E_UNSUPPORTED, "uyd_nms: max_det <= %d", kMaxDetCap);
-  if (max_nms > anchors) max_nms = anchors;
+  const bool multi = opt && opt->multi_label && nc > 1;  // Ultralytics: multi_label &= nc > 1
+  const bool filter = opt && opt->filter_classes;
+  const long long cands = multi ? (long long)anchors * nc : anchors;  // at most this many candidates per image
+  if (max_nms > cands) max_nms = (int)cands;
   UYD_REQUIRE(max_nms > 0, UYD_E_ARG, "uyd_nms: max_nms must be positive");
+  ClassMask cm{};
+  if (filter)  // ids outside [0, nc) match no class
+    for (int i = 0; i < opt->num_filter_classes; ++i) {
+      const int c = opt->filter_classes[i];
+      if (c >= 0 && c < nc) cm.w[c >> 5] |= 1u << (c & 31);
+    }
   float thr_f = (float)iou_thr;  // largest float <= the double threshold
   if ((double)thr_f > iou_thr) thr_f = nextafterf(thr_f, -INFINITY);
   if (int e = smem_optin(nms_image_kernel, sizeof(FusedSmem))) return e;
   nms_image_kernel<<<batch, kFThreads, sizeof(FusedSmem), (cudaStream_t)stream>>>(
-      y, nc, anchors, conf_thr, thr_f, max_nms, max_det, max_wh, conf_thr >= 0.f ? 1 : 0, out_det, out_idx, out_count);
+      y, nc, anchors, conf_thr, thr_f, max_nms, max_det, max_wh, conf_thr >= 0.f ? 1 : 0, out_det, out_idx, out_count,
+      (multi ? 2 : 0) | (filter ? 1 : 0), cm);
   UYD_CUDA(cudaGetLastError());
   return UYD_OK;
+}
+
+extern "C" int uyd_nms(uyd_ctx *ctx, const float *y, int batch, int nc, int anchors, float conf_thr, double iou_thr,
+                       int max_nms, int max_det, float max_wh, void *workspace, size_t workspace_bytes, float *out_det,
+                       int *out_idx, int *out_count, uyd_stream stream) {
+  (void)workspace; (void)workspace_bytes;
+  return uyd_nms_ex(ctx, y, batch, nc, anchors, conf_thr, iou_thr, max_nms, max_det, max_wh, nullptr, out_det, out_idx,
+                    out_count, stream);
 }
 
 extern "C" size_t uyd_nms_detections_workspace_bytes(int cap) { return cap > 0 ? 256 : 0; }  // kept for ABI stability: unused

@@ -13,6 +13,7 @@ from __future__ import annotations
 import ast
 import ctypes as C
 import math
+import operator
 import os
 from math import gcd
 from pathlib import Path
@@ -418,6 +419,27 @@ class Detect(nn.Module):
             heads.append(head if head is not None else Slice(-1, 0, self.no, f.h, f.w))
             a_off += f.h * f.w
         return heads
+
+
+def _class_ids(classes):
+    """Ultralytics' ``classes`` (None, an int or an iterable of ints) as a tuple of ints, or None."""
+    if classes is None:
+        return None
+    return tuple(operator.index(c) for c in ([classes] if isinstance(classes, int) else classes))
+
+
+def _nms_options(classes, multi_label: bool):
+    """``uyd_nms_options`` for Ultralytics' ``classes`` / ``multi_label``, or None at their defaults (plain ``uyd_nms``).
+    ``[]`` keeps nothing; ids outside [0, nc) match nothing."""
+    if classes is None and not multi_label:
+        return None
+    opt = _lib.NmsOptions(multi_label=1 if multi_label else 0)
+    if classes is not None:
+        # every id outside [0, 256] matches nothing: clamping keeps that and fits a C int
+        ids = [min(max(c, -1), 1 << 30) for c in _class_ids(classes)]
+        opt.num_filter_classes = len(ids)
+        opt.filter_classes = (C.c_int * max(1, len(ids)))(*ids)   # the struct keeps the array alive
+    return opt
 
 
 def _literal(a):
@@ -860,10 +882,13 @@ class UninaYoloB200(nn.Module):
 
     @torch.no_grad()
     def predict_camera(self, frames: torch.Tensor, size=None, norm=None, uv=None, conf: float = 0.25, iou: float = 0.7,
-                       max_det: int = 300, max_nms: int = 30000, letterbox: bool = False):
+                       max_det: int = 300, max_nms: int = 30000, letterbox: bool = False, *, classes=None,
+                       agnostic: bool = False, multi_label: bool = False):
         """``forward_camera`` + NMS: (det[B,max_det,6], count[B]) on the device.  With ``letterbox`` the rows are in
-        frame pixels (``scale_boxes`` + ``clip_boxes`` of the Ultralytics predictor, one launch)."""
-        det, cnt = self.nms(self.forward_camera(frames, size, norm, uv, letterbox), conf, iou, max_det, max_nms)
+        frame pixels (``scale_boxes`` + ``clip_boxes`` of the Ultralytics predictor, one launch).  ``classes``,
+        ``agnostic``, ``multi_label``: as in ``nms``."""
+        det, cnt = self.nms(self.forward_camera(frames, size, norm, uv, letterbox), conf, iou, max_det, max_nms,
+                            classes=classes, agnostic=agnostic, multi_label=multi_label)
         if letterbox:
             H, W = frames.shape[1:3]
             P.letterbox_boxes(det, cnt, H, W, *P.camera_extent(H, W, size, True))
@@ -877,10 +902,16 @@ class UninaYoloB200(nn.Module):
             self._nms_ws[dev] = ws
         return ws
 
-    def _nms_into(self, y, det, idx, cnt, ws, conf, iou, max_det, max_nms, max_wh) -> None:
-        """C call only (no allocation): safe inside CUDA-graph capture."""
+    def _nms_into(self, y, det, idx, cnt, ws, conf, iou, max_det, max_nms, max_wh, opt=None) -> None:
+        """C call only (no allocation): safe inside CUDA-graph capture.  ``opt``: ``_nms_options`` (None: uyd_nms)."""
         B, no, A = y.shape
         dev = y.device.index if y.device.index is not None else torch.cuda.current_device()
+        if opt is not None:
+            check(_lib.lib().uyd_nms_ex(_lib.context(dev), C.c_void_p(y.data_ptr()), B, no - 4, A, conf, iou, max_nms, max_det,
+                                        max_wh, C.byref(opt), C.c_void_p(det.data_ptr()),
+                                        C.c_void_p(idx.data_ptr()) if idx is not None else None, C.c_void_p(cnt.data_ptr()),
+                                        C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)), "uyd_nms_ex")
+            return
         check(_lib.lib().uyd_nms(_lib.context(dev), C.c_void_p(y.data_ptr()), B, no - 4, A, conf, iou, max_nms, max_det,
                                  max_wh, C.c_void_p(ws.data_ptr()), ws.numel(), C.c_void_p(det.data_ptr()),
                                  C.c_void_p(idx.data_ptr()) if idx is not None else None, C.c_void_p(cnt.data_ptr()),
@@ -888,8 +919,13 @@ class UninaYoloB200(nn.Module):
 
     @torch.no_grad()
     def nms(self, y: torch.Tensor, conf: float = 0.25, iou: float = 0.7, max_det: int = 300, max_nms: int = 30000,
-            max_wh: float = 7680.0, return_index: bool = False):
-        """Ultralytics ``non_max_suppression`` on ``y[B,4+nc,A]`` -> (det[B,max_det,6], count[B])."""
+            max_wh: float = 7680.0, return_index: bool = False, *, classes=None, agnostic: bool = False,
+            multi_label: bool = False):
+        """Ultralytics ``non_max_suppression`` on ``y[B,4+nc,A]`` -> (det[B,max_det,6], count[B]).
+        ``classes``: keep only these class ids (an int or a list; ``[]`` keeps nothing), filtered before the
+        ``max_nms`` truncation and the NMS.  ``agnostic``: NMS across classes (``max_wh`` 0).  ``multi_label``: every
+        (anchor, class) pair with a score above ``conf`` is a candidate (what ``model.val`` runs), not only the best
+        class of each anchor; ``return_index`` then gives the anchor of each row."""
         assert y.is_cuda and y.dtype == torch.float32 and y.is_contiguous()
         B, no, A = y.shape
         dev = y.device.index if y.device.index is not None else torch.cuda.current_device()
@@ -898,17 +934,18 @@ class UninaYoloB200(nn.Module):
         det = torch.empty(B, max_det, 6, dtype=torch.float32, device=y.device)
         idx = torch.empty((B, max_det), dtype=torch.int32, device=y.device) if return_index else None
         cnt = torch.empty(B, dtype=torch.int32, device=y.device)
-        self._nms_into(y, det, idx, cnt, ws, conf, iou, max_det, max_nms, max_wh)
+        self._nms_into(y, det, idx, cnt, ws, conf, iou, max_det, max_nms, 0.0 if agnostic else max_wh,
+                       _nms_options(classes, multi_label))
         return (det, cnt, idx) if return_index else (det, cnt)
 
     # batches up to this size replay a captured CUDA graph (the ~70 launches of a step are
     # launch-latency-bound below it); larger batches are launched directly.
     GRAPH_MAX_BATCH = 8
 
-    def _graph_for(self, x: torch.Tensor, conf, iou, max_det, max_nms):
+    def _graph_for(self, x: torch.Tensor, conf, iou, max_det, max_nms, classes=None, agnostic=False, multi_label=False):
         B, _, H, W = x.shape
         dev = x.device.index if x.device.index is not None else torch.cuda.current_device()
-        key = (dev, B, H, W, x.dtype, float(conf), float(iou), int(max_det), int(max_nms))
+        key = (dev, B, H, W, x.dtype, float(conf), float(iou), int(max_det), int(max_nms), _class_ids(classes), bool(agnostic), bool(multi_label))
         g = self._graphs.get(key)
         if g is not None:
             return g
@@ -918,11 +955,12 @@ class UninaYoloB200(nn.Module):
         det = torch.zeros(B, max_det, 6, dtype=torch.float32, device=x.device)
         cnt = torch.zeros(B, dtype=torch.int32, device=x.device)
         ws = torch.empty(int(_lib.lib().uyd_nms_workspace_bytes(B, A)), dtype=torch.uint8, device=x.device)
+        opt = _nms_options(classes, multi_label)   # read at launch: the captured kernel holds the class mask by value
 
         def body():
             det.zero_()
             self._decoded_into(xs, y)
-            self._nms_into(y, det, None, cnt, ws, conf, iou, max_det, max_nms, 7680.0)
+            self._nms_into(y, det, None, cnt, ws, conf, iou, max_det, max_nms, 0.0 if agnostic else 7680.0, opt)
 
         xs.copy_(x)
         side = torch.cuda.Stream(device=x.device)
@@ -940,31 +978,37 @@ class UninaYoloB200(nn.Module):
 
     @torch.no_grad()
     def predict_batched(self, x: torch.Tensor, conf: float = 0.25, iou: float = 0.7, max_det: int = 300,
-                        max_nms: int = 30000, graph: bool | None = None):
+                        max_nms: int = 30000, graph: bool | None = None, *, classes=None, agnostic: bool = False,
+                        multi_label: bool = False):
         """Forward + decode + NMS, everything left on the device: (det[B,max_det,6], count[B]).
-        ``graph`` (default: batch <= GRAPH_MAX_BATCH) replays the whole step as one CUDA graph."""
+        ``graph`` (default: batch <= GRAPH_MAX_BATCH) replays the whole step as one CUDA graph.  ``classes``,
+        ``agnostic``, ``multi_label``: as in ``nms``; ``model.val``'s NMS is ``conf=0.001, iou=0.7, multi_label=True``."""
         x = self._prep(x)
         if graph is None:
             graph = x.shape[0] <= self.GRAPH_MAX_BATCH and os.environ.get("UYD_NO_GRAPH", "0") != "1"
         if graph:
             with torch.cuda.device(x.device):   # capture and replay on the frames' device, whatever the caller's current one is
-                g, xs, det, cnt, _ = self._graph_for(x, conf, iou, max_det, max_nms)
+                g, xs, det, cnt, _ = self._graph_for(x, conf, iou, max_det, max_nms, classes, agnostic, multi_label)
                 xs.copy_(x)
                 g.replay()
                 return det.clone(), cnt.clone()
         y = self.forward(x, raw_heads=False)
-        return self.nms(y, conf, iou, max_det, max_nms)
+        return self.nms(y, conf, iou, max_det, max_nms, classes=classes, agnostic=agnostic, multi_label=multi_label)
 
     @torch.no_grad()
-    def predict(self, x: torch.Tensor, conf: float = 0.25, iou: float = 0.7, max_det: int = 300, max_nms: int = 30000):
-        """Per-image ``[N_i, 6]`` tensors ``(x1,y1,x2,y2,conf,cls)`` like ``result.boxes.data``."""
-        det, cnt = self.predict_batched(x, conf, iou, max_det, max_nms)
+    def predict(self, x: torch.Tensor, conf: float = 0.25, iou: float = 0.7, max_det: int = 300, max_nms: int = 30000, *,
+                classes=None, agnostic: bool = False, multi_label: bool = False):
+        """Per-image ``[N_i, 6]`` tensors ``(x1,y1,x2,y2,conf,cls)`` like ``result.boxes.data``; ``classes`` and
+        ``agnostic`` are ``YOLO.predict``'s ``classes=`` / ``agnostic_nms=`` (see ``nms``)."""
+        det, cnt = self.predict_batched(x, conf, iou, max_det, max_nms, classes=classes, agnostic=agnostic,
+                                        multi_label=multi_label)
         counts = cnt.tolist()
         return [det[b, :n] for b, n in enumerate(counts)]
 
     @torch.no_grad()
     def predict_stream(self, batches, conf: float = 0.25, iou: float = 0.7, max_det: int = 300, max_nms: int = 30000,
-                       to_host: bool = True, camera: str | None = None, size=None, norm=None, letterbox: bool = False):
+                       to_host: bool = True, camera: str | None = None, size=None, norm=None, letterbox: bool = False, *,
+                       classes=None, agnostic: bool = False, multi_label: bool = False):
         """Generator form of ``predict`` (the reference consumes ``YOLO.predict(..., stream=True)``,
         train.py:396-423): ``batches`` yields host frame batches ``[B,3,H,W]`` (uint8 or float, ideally
         pinned).  Batch i+1 is copied host->device on a copy stream while batch i computes, so a
@@ -979,7 +1023,7 @@ class UninaYoloB200(nn.Module):
         ``[B, 3H/2, W]`` (the Y rows followed by the interleaved UV rows: 1.5 bytes per pixel over PCIe instead of 3),
         ``"bgra"`` = uint8 ``[B, H, W, 4]`` (resampled to ``size`` when given); ``norm`` as in ``forward_camera``.
         ``letterbox`` (``camera="bgra"`` only): the frames are letterboxed as in ``forward_camera`` and the rows come
-        back in frame pixels."""
+        back in frame pixels.  ``classes``, ``agnostic``, ``multi_label``: as in ``nms``."""
         if camera not in (None, "nv12", "bgra"):
             raise ValueError("camera must be None, 'nv12' or 'bgra'")
         if letterbox and camera != "bgra":
@@ -1064,7 +1108,8 @@ class UninaYoloB200(nn.Module):
                 y = self.forward_camera(xin, size, norm, None, letterbox)
             elif r.n <= self.GRAPH_MAX_BATCH and os.environ.get("UYD_NO_GRAPH", "0") != "1":
                 y = None   # small batches replay the whole step as one CUDA graph
-                r.det, r.cnt = self.predict_batched(xin, conf, iou, max_det, max_nms)
+                r.det, r.cnt = self.predict_batched(xin, conf, iou, max_det, max_nms, classes=classes, agnostic=agnostic,
+                                                    multi_label=multi_label)
             else:
                 y = self.forward(xin, raw_heads=False)
             s.free.record(main_s)
@@ -1073,7 +1118,8 @@ class UninaYoloB200(nn.Module):
                 post_s.wait_event(r.fwd)
                 if y is not None:
                     y.record_stream(post_s)
-                    r.det, r.cnt = self.nms(y, conf, iou, max_det, max_nms)
+                    r.det, r.cnt = self.nms(y, conf, iou, max_det, max_nms, classes=classes, agnostic=agnostic,
+                                            multi_label=multi_label)
                     if letterbox:
                         h0, w0 = xin.shape[1:3]
                         P.letterbox_boxes(r.det, r.cnt, h0, w0, *P.camera_extent(h0, w0, size, True))
